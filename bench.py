@@ -18,9 +18,13 @@ e2e    : the same through the C ABI with HOST buffers: b7_gp_fit_sharded (X, y, 
 multi  : one process per GPU (torchrun); everything that crosses GPUs runs inside libbot7_b200.so (b7_comm_init_rank,
          b7_gp_fit_sharded, b7_acq_score_multi: NCCL over NVLink); torch.distributed (gloo) only carries the 128-byte
          NCCL id, the barriers and the max over ranks of the timings.
-Launch : python bench.py --gpus N --steps K --warmup W [--config headline|c1|c2|c3|c4|c5] [--scaling weak|strong]
+Launch : python bench.py --gpus N --steps K --warmup W [--config headline|c1|c2|c3|c4|c5] [--scaling weak|strong] [--dump-outputs DIR]
          python bench.py --impl reference ...     (CPU arm: the oracle port on the host cores, same config)
 Prints ONE JSON line on rank 0; exits 3 if the two posterior paths select different candidates.
+--dump-outputs DIR: also writes what the last timed step returned as DIR/<name>.npy, so that two builds run with the same
+         arguments can be compared output for output: the combined best score, argmax and NaN count (rank 0) and the score vector
+         of every rank's shard (scores.npy on one GPU, scores_rank<r>.npy on several).  The scores come from one more step after
+         the timed window, on the same inputs, which must return the timed step's result bit for bit.
 """
 import argparse
 import ctypes as C
@@ -36,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True            # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 N_OBS, DIMS, S_DRAWS = 4096, 6, 32
 SMS = 148
@@ -283,6 +288,35 @@ def slices_bytes_per_draw(Np):
     return 4 * P * (P + 1) * 57344
 
 
+# ------------------------------------------------------------------ outputs
+
+DUMP_MAX_VALUES = 1 << 21                 # per array: 16 MB of float64, so a dump stays well under 64 MB
+
+
+def dump_outputs(out_dir, arrays, max_values=DUMP_MAX_VALUES):
+    """arrays: name -> values, written as out_dir/<name>.npy in float64.  An array with more than max_values elements is
+    stored as a fixed, seeded sample of them, the sampled positions beside it as <name>_rows.npy: the same elements every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).reshape(-1)
+        if a.size > max_values:
+            rows = np.sort(np.random.default_rng(0).choice(a.size, max_values, replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dump_last_step(args, world, rank, res, step, names):
+    """--dump-outputs: `res` is what the last timed step returned, `step(True)` repeats it outside the timed window and also returns
+    this rank's score vector (last element).  names: the output names of res.  Every rank takes part (the step may hold collectives)."""
+    again = step(True)
+    if not np.array_equal(np.array(again[:len(names)], float), np.array(res[:len(names)], float), equal_nan=True):
+        raise RuntimeError(f"--dump-outputs: the repeated step returned {again[:len(names)]}, the timed step {res[:len(names)]}")
+    arrays = {n: [v] for n, v in zip(names, res)} if rank == 0 else {}
+    arrays["scores" if world == 1 else f"scores_rank{rank}"] = again[-1]
+    dump_outputs(args.dump_outputs, arrays, DUMP_MAX_VALUES // world)     # at most 32 MB over all ranks
+
+
 # ------------------------------------------------------------------ GPU arm
 
 _REAL_STDOUT = None
@@ -310,7 +344,12 @@ def main():
     ap.add_argument("--e2e-candidates", type=int, default=None, help="candidates per GPU of the end-to-end leg (default: 2^20 at the headline, else the step's)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-path", action="store_true", help="skip the FP64 DMMA path that the 1-GPU headline run times beside the default one")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -419,17 +458,17 @@ def main():
 
     state = {"gps": gps}
 
-    def step():
+    def step(want_scores=False):
+        """-> (best, argmax, argmax_original, nan_count, scores of this rank's shard or None), as comm.acq_score returns them."""
         if strong:                         # fit + exchange inside the step
             comm.free_fit(state["gps"])
             state["gps"] = comm.fit(Xo, y, hyp)[0]
-        b_, a_, ao_, n_, _ = comm.acq_score(state["gps"], grids_, kind, tradeoff, 0, -1.0, fmin)
-        return b_, ao_, n_
+        return comm.acq_score(state["gps"], grids_, kind, tradeoff, 0, -1.0, fmin, want_scores=want_scores)
 
     def timed(path, warmup, steps, profiled):
         """`steps` timed steps; returns (device ms per step (max over ranks), wall ms, launches (sum over ranks), stage times, clocks,
-        result).  profiled = False: the number that counts (no per-stage synchronisation, K* of draw s + 1 runs under the posterior pass
-        of draw s); profiled = True: per-launch CUDA-event times for the roofline (every stage synchronises)."""
+        result of the last step).  profiled = False: the number that counts (no per-stage synchronisation, K* of draw s + 1 runs under
+        the posterior pass of draw s); profiled = True: per-launch CUDA-event times for the roofline (every stage synchronises)."""
         if ctx.posterior_path() != path:
             ctx.set_posterior_path(path)
             if not strong:                 # the resident factors were exchanged in the other path's form
@@ -467,6 +506,8 @@ def main():
         _, _, _, o_st, _, _ = timed(other_path, 0, 1, True)
         other = (o_ms, o_launches, o_clk, o_res, o_st)
     ms_per_step, wall_ms, launches, _, clocks, res = timed(default_path, args.warmup, args.steps, False)
+    if args.dump_outputs:
+        dump_last_step(args, world, rank, res, step, ["best", "argmax", "argmax_original", "nan_count"])
     prof_steps = 1 if strong else 2
     prof_ms, _, _, st, _, _ = timed(default_path, 0, prof_steps, True)
     value = M_total / (ms_per_step * 1e-3)
@@ -595,7 +636,7 @@ def main():
         "gpu_launches": int(launches), "wall_ms_per_step": wall_ms,
         "clocks": clocks, "roofline": roofline, "stages": stages, "peaks": pk,
         "posterior_path": path_name[default_path],
-        "result": {"best": res[0], "global_index": res[1], "nan_count": res[2]},
+        "result": {"best": res[0], "global_index": res[2], "nan_count": res[3]},
     }
     if e2e_step_batch:
         line["e2e_step_batch"] = e2e_step_batch
@@ -603,7 +644,7 @@ def main():
         o_ms, o_launches, o_clk, o_res, o_st = other
         line["other_path"] = {"posterior_path": path_name[other_path], "value": M_total / (o_ms * 1e-3), "unit": UNIT, "ms_per_step": o_ms,
                               "gpu_launches": int(o_launches), "roofline": posterior_roofline(other_path, o_st, o_ms, 1), "clocks": o_clk,
-                              "same_argmax": bool(o_res[1] == res[1]), "best_rel_diff": abs(o_res[0] - res[0]) / abs(res[0]) if res[0] else None}
+                              "same_argmax": bool(o_res[2] == res[2]), "best_rel_diff": abs(o_res[0] - res[0]) / abs(res[0]) if res[0] else None}
     if not args.no_cpu_baseline and world == 1:
         c = cpu_sample(cfg)
         line["cpu_baseline"] = {"value": c["value"], "unit": UNIT, "cores": c["cores"], "kind": "port", "sample": c["sample"],
@@ -638,12 +679,14 @@ def bench_dngo(args, cfg, comm, ctx, L, lib, models, parallel, dist, pk, Xo, y, 
     fit_ms = ctx.stage_times()["blr"][0]
     ctx.set_profiling(False)
 
-    def step():
+    def step(want_scores=False):
+        """-> (best, global argmax_original, nan_count, scores of this rank's shard or None)."""
         am, amo, best, nn = C.c_int64(), C.c_int64(), C.c_double(), C.c_int64()
-        L.check(lib.b7_blr_score(blr.handle, feats.handle, EI, 0.0, 0, -1.0, fmin, None, C.byref(am), C.byref(amo), C.byref(best), C.byref(nn)),
-                "b7_blr_score")
+        sc = np.empty(cnt) if want_scores else None
+        L.check(lib.b7_blr_score(blr.handle, feats.handle, EI, 0.0, 0, -1.0, fmin, L.dptr(sc), C.byref(am), C.byref(amo), C.byref(best),
+                                 C.byref(nn)), "b7_blr_score")
         gi = amo.value + row0 if amo.value > 0 else 0
-        return parallel.allgather_argmax(best.value, gi, nn.value) if dist else (best.value, gi, nn.value)
+        return (*(parallel.allgather_argmax(best.value, gi, nn.value) if dist else (best.value, gi, nn.value)), sc)
 
     def timed(warmup, steps, profiled):
         ctx.set_profiling(profiled)
@@ -669,6 +712,8 @@ def bench_dngo(args, cfg, comm, ctx, L, lib, models, parallel, dist, pk, Xo, y, 
         return dev / steps, wall / steps, n_l, st_, clk_.summary(), r
 
     ms_per_step, wall_ms, launches, _, clocks, res = timed(args.warmup, args.steps, False)
+    if args.dump_outputs:
+        dump_last_step(args, world, rank, res, step, ["best", "argmax_original", "nan_count"])
     _, _, _, st, _, _ = timed(0, 3, True)
     blr_ms = st["blr"][0] / 3
     e2e_times = []

@@ -1,4 +1,4 @@
-"""Golden vectors produced by EXECUTING the reference's own Lua (read-only tree /root/reference) under tools/minilua.
+"""Golden vectors produced by EXECUTING the reference's own Lua (a read-only checkout named by BOT7_REFERENCE) under tools/minilua.
 
 The image has no Lua runtime and the reference holds no test vectors, so until now the oracle was pinned by hand-traced known
 answers only.  tools/minilua (a Lua 5.1 interpreter with a numpy-backed Torch7 tensor stand-in, written for this repository)
@@ -11,7 +11,7 @@ What this is and is not: the control flow and every arithmetic operation are the
 underneath is not LuaJIT + TH but Python floats + numpy (IEEE doubles, element-wise operations in storage order; `exp` is
 numpy's, which may differ from glibc's in the last ulp).  torch.potrf is LAPACK dpotrf through scipy, as TH's is.
 
-Run (only where /root/reference exists):  python tests/golden/make_ref_exec.py
+Run (with a checkout of the reference):  BOT7_REFERENCE=<bot7 checkout> python tests/golden/make_ref_exec.py
 """
 import io
 import os
@@ -25,12 +25,14 @@ from minilua import Interpreter, LuaError  # noqa: E402
 from minilua import torch7  # noqa: E402
 from minilua.interp import LuaTable  # noqa: E402
 
-REF = "/root/reference"
+REF = os.environ.get("BOT7_REFERENCE", "")         # a checkout of the reference bot7 Lua source, if any
 OUT = os.path.join(ROOT, "tests", "golden", "ref_exec.npz")
 
 
 def reference_runtime(seed=0):
     """An interpreter with the reference's utils / grids / scores / benchmarks modules loaded from the reference tree."""
+    if not os.path.isdir(REF):
+        raise RuntimeError("set BOT7_REFERENCE to a checkout of the reference bot7 source")
     out = io.StringIO()
     I = Interpreter(stdout=out)
     T = torch7.install(I, seed)
@@ -237,7 +239,7 @@ return score, idx, torch.Tensor(order)
 
 if __name__ == "__main__":
     if not os.path.isdir(REF):
-        sys.exit("reference tree not present: nothing to execute")
+        sys.exit("set BOT7_REFERENCE to a checkout of the reference bot7 source: nothing to execute")
     G, printed = generate()
     if os.environ.get("REF_EXEC_FAST"):
         OUT = "/tmp/ref_exec_fast.npz"                   # the debugging subset never replaces the committed file

@@ -581,10 +581,34 @@ return out[1], out[2], out[3], out[4]
 
 # ---------------------------------------------------------------------------------- the interpreter on the reference's own Lua (CPU)
 
-REF = "/root/reference"
+REF = os.environ.get("BOT7_REFERENCE", "")         # a checkout of the reference bot7 Lua source, if any
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+def _lua_spec_chain(rt, speculative, width):
+    """120 draws of a correlated 2-D Gaussian from seed 11 in `rt`, by lua/bot7_b200/sampler_spec.lua (batch width `width`) or,
+    not speculative, by bot7.samplers.slice (the reference's, loaded into `rt` by the caller): alternately narrow brackets that
+    step out and wide ones that shrink.  -> (chain 120 x 2, density evaluations, batched calls, the generator's next draw)."""
+    rt.set_global("SPEC", speculative)
+    rt.set_global("WIDTH", width)
+    r = rt.run(r"""
+local evals, calls = 0, 0
+local function logp1(x, a) return -0.5 * (x[1] ^ 2 / a.v1 + x[2] ^ 2 / a.v2 + 0.3 * x[1] * x[2]) end
+local function f(x, a) evals = evals + 1; return logp1(x[1], a) end
+local function fb(P, a) calls = calls + 1; local o = torch.Tensor(P:size(1)); for i = 1, P:size(1) do evals = evals + 1; o[i] = logp1(P[i], a) end; return o end
+local sampler = SPEC and require('bot7_b200.sampler_spec')() or bot7.samplers.slice()
+local out, x = torch.Tensor(120, 2), torch.Tensor{{0.3, -0.2}}
+for i = 1, 120 do
+  local opt = {nSamples = 1, width = (i % 2 == 0) and 0.05 or 6.0}        -- narrow brackets step out, wide ones shrink
+  if SPEC then x = sampler(fb, x, opt, {v1 = 1.0, v2 = 4.0}, WIDTH) else x = sampler(f, x, opt, {v1 = 1.0, v2 = 4.0}) end
+  out[i]:copy(x[1])
+end
+return out, evals, calls, torch.rand(1)[1]
+""")
+    rt.close()
+    return r[0].a, r[1], r[2], r[3]
+
+
+@pytest.mark.skipif(not os.path.isdir(REF), reason="bot7 reference source not found (set BOT7_REFERENCE to a checkout)")
 def test_interpreter_runs_the_reference_slice_sampler_unchanged():
     """Validation of the interpreter and the tensor stand-in on code that was written for the real runtime: the reference's
     samplers/abstract.lua, samplers/slice.lua and utils/tensor.lua are loaded from the read-only reference tree, unmodified, and
@@ -641,7 +665,7 @@ return out, evals, gibbs, torch.type(sampler)
     assert "Error" not in out.getvalue()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="bot7 reference source not found (set BOT7_REFERENCE to a checkout)")
 @pytest.mark.parametrize("width", [1, 3, 4, 8])
 def test_lua_speculative_sampler_walks_the_executed_reference_chain(width):
     """lua/bot7_b200/sampler_spec.lua (batched density evaluations, generator rewound after discarded speculation) against
@@ -656,24 +680,7 @@ def test_lua_speculative_sampler_walks_the_executed_reference_chain(width):
         I.G.get("package").get("loaded").set("bot7.utils", I.G.get("bot7").get("utils"))
         I.run_file(os.path.join(REF, "samplers", "abstract.lua"))
         I.run_file(os.path.join(REF, "samplers", "slice.lua"))
-        I.G.set("SPEC", speculative)
-        I.G.set("WIDTH", width)
-        r = I.run(r"""
-local evals, calls = 0, 0
-local function logp1(x, a) return -0.5 * (x[1] ^ 2 / a.v1 + x[2] ^ 2 / a.v2 + 0.3 * x[1] * x[2]) end
-local function f(x, a) evals = evals + 1; return logp1(x[1], a) end
-local function fb(P, a) calls = calls + 1; local o = torch.Tensor(P:size(1)); for i = 1, P:size(1) do evals = evals + 1; o[i] = logp1(P[i], a) end; return o end
-local sampler = SPEC and require('bot7_b200.sampler_spec')() or bot7.samplers.slice()
-local out, x = torch.Tensor(120, 2), torch.Tensor{{0.3, -0.2}}
-for i = 1, 120 do
-  local opt = {nSamples = 1, width = (i % 2 == 0) and 0.05 or 6.0}        -- narrow brackets step out, wide ones shrink
-  if SPEC then x = sampler(fb, x, opt, {v1 = 1.0, v2 = 4.0}, WIDTH) else x = sampler(f, x, opt, {v1 = 1.0, v2 = 4.0}) end
-  out[i]:copy(x[1])
-end
-return out, evals, calls, torch.rand(1)[1]
-""")
-        rt.close()
-        return r[0].a, r[1], r[2], r[3]
+        return _lua_spec_chain(rt, speculative, width)
     ref, ref_evals, _, ref_next = chain(False)
     got, evals, calls, nxt = chain(True)
     assert np.array_equal(got, ref)                       # the same chain, bit for bit
@@ -681,3 +688,28 @@ return out, evals, calls, torch.rand(1)[1]
     assert calls < ref_evals                              # in fewer sequential (device) calls
     if width >= 4:
         assert calls < 0.5 * ref_evals
+
+
+@pytest.mark.parametrize("width", [1, 3, 4, 8])
+def test_lua_speculative_sampler_walks_the_python_twin_chain(width):
+    """lua/bot7_b200/sampler_spec.lua against bot7_b200/samplers.py:slice, the Python restatement of samplers/slice.lua, on the
+    chain of the test above and without the reference tree: from the same seed the two walk the same chain (to the rounding of
+    the direction's norm: BLAS dot in numpy vs a sum of squares), draw the same random numbers (the generator is left in the same
+    state) and the speculative one needs fewer sequential density calls."""
+    sys.path.insert(0, ROOT)
+    from bot7_b200 import samplers
+    got, _, calls, nxt = _lua_spec_chain(GlueRuntime(seed=11, fixture=False), True, width)
+    rng, evals = np.random.default_rng(11), [0]
+
+    def logp(x, a):
+        evals[0] += 1
+        return -0.5 * (x[0, 0] ** 2 / a["v1"] + x[0, 1] ** 2 / a["v2"] + 0.3 * x[0, 0] * x[0, 1])
+    tw, x, chain = samplers.slice(), np.array([[0.3, -0.2]]), np.empty((120, 2))
+    for i in range(1, 121):
+        x = tw(logp, x, {"nSamples": 1, "width": 0.05 if i % 2 == 0 else 6.0}, {"v1": 1.0, "v2": 4.0}, rng)
+        chain[i - 1] = x[0]
+    assert np.allclose(got, chain, rtol=0.0, atol=1e-12)
+    assert nxt == rng.random()
+    assert calls < evals[0]
+    if width >= 4:
+        assert calls < 0.5 * evals[0]

@@ -3,7 +3,7 @@ tests/test_lua_reference_loop.py.  Checked here, without running anything: the g
 call sites and well-formed:
 
 * every method the reference calls on the model / score / grid / sampler objects of the accelerated path
-  (extracted from /root/reference when it is present, otherwise from the committed list below, which was extracted
+  (extracted from the reference named by BOT7_REFERENCE when it is present, otherwise from the committed list below, which was extracted
   from it) is defined by the replacement class, or inherited from the reference parent it subclasses;
 * every C symbol the glue calls through `B.C.` is declared in include/bot7_b200.h (and therefore in the generated cdef);
 * block keywords balance (the first, parser-free check) and, with tools/lua_check.py, the full grammar, every name, every
@@ -16,7 +16,7 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LUA = os.path.join(ROOT, "lua", "bot7_b200")
-REF = "/root/reference"
+REF = os.environ.get("BOT7_REFERENCE", "")         # a checkout of the reference bot7 Lua source, if any
 
 # method names the reference calls on `self.model` / `model` in the files of the path (SURVEY section 8b):
 #   bots/abstract.lua:148 init; bots/bayesopt.lua:65,68,74,75 class, sample_hypers, parse_hypers;
@@ -41,7 +41,7 @@ def defined_methods(text, cls):
 
 def test_reference_call_sites_match_the_committed_list():
     if not os.path.isdir(REF):
-        pytest.skip("reference tree not present (GPU box)")
+        pytest.skip("bot7 reference source not found (set BOT7_REFERENCE to a checkout)")
     called = set()
     for f in CALL_SITES:
         src = strip_comments(open(os.path.join(REF, f)).read())
@@ -163,7 +163,7 @@ def test_self_method_calls_resolve(name):
 def test_checker_parses_the_whole_reference_tree():
     """Validation of the checker itself: all of the reference's Lua (5 k lines written for the real interpreter) parses."""
     if not os.path.isdir(REF):
-        pytest.skip("reference tree not present (GPU box)")
+        pytest.skip("bot7 reference source not found (set BOT7_REFERENCE to a checkout)")
     n = 0
     for dirpath, _, files in os.walk(REF):
         for f in files:

@@ -4,7 +4,7 @@ loaded UNMODIFIED from the read-only reference tree under tools/minilua, `requir
 classes, and whole Bayesian-optimisation experiments run -- BASELINE.json's config 1 (examples/run_benchmark.lua: Branin-Hoo,
 bayesopt EI, GP ARD-SE, Sobol candidates) through the reference's own example script.
 
-This can only run where the reference tree is (the build container), which has no GPU; the library has no CPU path.  So the
+This needs a checkout of the reference (named by BOT7_REFERENCE) and runs without a GPU; the library has no CPU path.  So the
 glue's `ffi.load` is answered by tests/fake_b7_lib.py, an oracle-backed object with the C ABI's signatures.  What is under test
 is therefore the PROTOCOL between the reference's classes, the glue and the C ABI -- constructor chains, which object owns which
 field, compacted vs original numbering across `utils.tensor.steal` and `b7_grid_remove`, handle lifetimes -- in the one setting
@@ -20,7 +20,7 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("BOT7_REFERENCE", "")         # a checkout of the reference bot7 Lua source, if any
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from minilua import Interpreter, LuaError  # noqa: E402,F401
@@ -29,7 +29,7 @@ from minilua import torch7  # noqa: E402
 from minilua.harness import LUA_DIR  # noqa: E402
 from minilua.interp import LuaTable  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="bot7 reference source not found (set BOT7_REFERENCE to a checkout)")
 
 CMDLINE = r"""
 local Cmd = torch.class('torch.CmdLine')

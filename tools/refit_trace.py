@@ -1,6 +1,7 @@
 import os, sys, time
 import numpy as np
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/oracle")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import b7_oracle as o
 from bot7_b200 import _lib as L, models
 N, d = 4096, 6
