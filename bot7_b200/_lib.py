@@ -70,6 +70,8 @@ SIGNATURES = {
     "b7_score_moments": (_i, [_p, _i, _dp, _dp, _i, _l, _d, _i, _d, _d, _dp, _lp, _dp, _lp]),
     "b7_mlp_features": (_i, [_p, _p, _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _i, C.POINTER(_p)]),
     "b7_blr_fit": (_i, [_p, _dp, _dp, _i, _i, _dp, _i, C.POINTER(_p), _ip]),
+    "b7_blr_refit": (_i, [_p, _dp, _i, _ip, _dp]),
+    "b7_blr_num_draws": (_i, [_p]),
     "b7_blr_predict": (_i, [_p, _i, _dp, _l, _dp, _dp]),
     "b7_blr_score": (_i, [_p, _p, _i, _d, _i, _d, _d, _dp, _lp, _lp, _dp, _lp]),
     "b7_dngo_score": (_i, [_p, _p, _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _i, _i, _d, _i, _d, _d, _dp, _lp, _lp, _dp, _lp]),

@@ -122,6 +122,19 @@ struct b7_blr {
   double* w = nullptr;     // device S x D
   double* par = nullptr;   // device S x 4: alpha_p, beta, m, 1/beta
   std::vector<double> par_host;
+  bool ready = true;       // Linv / w belong to par (false after a B7_FIT_LOGML_ONLY refit)
+  // resident for b7_blr_refit (the log evidence the slice sampler evaluates, blr.cu)
+  double* Z = nullptr;         // device N x D
+  double* y = nullptr;         // device N
+  double* partial = nullptr;   // device gram_blocks x (D*D + 2D): gram_kernel's per-block partials
+  int gram_blocks = 0;
+  double* gram = nullptr;      // device D*D + 2D: the partials summed in block order (first refit)
+  double* hyp = nullptr;       // device S x 3: the rows of the last refit
+  double* ev_w = nullptr;      // device S x D: w of the evidence pass
+  double* ev_stat = nullptr;   // device S x 2: sum log (L_A)_ii, |w|^2
+  double* ev_res = nullptr;    // device S x res_blocks: partial sums of |r - Z0 w|^2
+  double* ev_out = nullptr;    // device S: log p(y | row)
+  int* ev_info = nullptr;      // device 2S: evidence factor, predictor factor
 };
 
 // sharded fit (multi.cu): before / after the exchange of the per-draw state (api.cu)

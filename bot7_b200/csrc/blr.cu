@@ -10,6 +10,8 @@
 // fit:   gram_kernel accumulates per-block partial sums of Z0^T Z0, Z0^T y, Z0^T 1 in registers
 //        (fixed row partition, partials added in block order => deterministic), blr_finish_kernel
 //        factors and inverts the D x D system in shared memory, one CTA per (alpha_p, beta) draw.
+// refit: the partials, Z0 and y stay on the device; new rows give the log evidence (blr_evidence_kernel +
+//        blr_residual_kernel, the slice sampler's density) and, on request, a new predictor through blr_finish_kernel.
 // score: one thread per candidate keeps its D features in registers (instantiated for D rounded up
 //        to a multiple of 8, D <= 64), L^-1 sits in shared memory and is read as warp broadcasts;
 //        the pass reads 8D bytes per candidate once (tile staged through shared memory so the
@@ -138,6 +140,163 @@ blr_finish_kernel(const double* __restrict__ partial, int n_blocks, int D, const
     Linv[(long long)s * D * D + e] = (k <= i) ? X[i * ld + k] : 0.0;
   }
   if (tid == 0) info[s] = my_info;
+}
+
+// ---- log evidence of the BLR head for S rows (b7_blr_refit) --------------------------------------------------
+//   log p(y | h) = D/2 log alpha_p + N/2 log beta - E - sum_i log (L_A)_ii - N/2 log 2 pi,
+//   E = beta/2 |r - Z0 w|^2 + alpha_p/2 |w|^2,  r = y - m.
+// E is evaluated as written, by a residual pass over the resident Z0 (blr_residual_kernel): E is the minimum over w of
+// that quadratic, so an error in w enters E at second order only.  The shortcut E = (beta r^T r - |L_A^-1 beta Z0^T r|^2) / 2
+// subtracts two numbers of size beta r^T r and loses their common digits (at beta = 1e4, N = 20 000 that is 1e-8 relative
+// to the result when the features explain y well).  Every draw is computed by its own CTA / its own registers, so a draw's
+// result does not depend on the other rows of the launch.
+
+// gram[o] = sum_p partial[p][o], in block order: the sums blr_finish_kernel forms, so A below has the same bits
+__global__ void blr_gram_reduce_kernel(const double* __restrict__ partial, int n_blocks, int n_out, double* __restrict__ gram) {
+  const int o = blockIdx.x * blockDim.x + threadIdx.x;
+  if (o >= n_out) return;
+  double a = 0.0;
+  for (int p = 0; p < n_blocks; ++p) a += partial[(long long)p * n_out + o];
+  gram[o] = a;
+}
+
+// One CTA per draw: A = beta G + alpha_p I, L_A = chol(A) in shared memory (no inverse), u = L_A^-1 beta Z0^T r by
+// forward substitution, w = L_A^-T u by back substitution.  Writes w[s], stat[s] = (sum log (L_A)_ii, |w|^2), info[s]
+// (first failing pivot; a non-finite pivot fails too).
+__global__ void __launch_bounds__(256)
+blr_evidence_kernel(const double* __restrict__ gram, int D, const double* __restrict__ par, double* __restrict__ w_out,
+                    double* __restrict__ stat, int* __restrict__ info) {
+  extern __shared__ double sh[];
+  const int ld = D + 1, s = blockIdx.x, tid = threadIdx.x, n_out = D * D + 2 * D;
+  double* A = sh;                 // D x ld : lower = L_A
+  double* b = A + D * ld;         // D
+  double* t1 = b + D;             // D
+  const double alpha_p = par[s * 4 + 0], beta = par[s * 4 + 1], m = par[s * 4 + 2];
+  for (int o = tid; o < n_out; o += blockDim.x) {
+    const double a = gram[o];
+    if (o < D * D) {
+      const int i = o / D, j = o % D;
+      A[i * ld + j] = beta * a + (i == j ? alpha_p : 0.0);
+    } else if (o < D * D + D) b[o - D * D] = a;
+    else t1[o - D * D - D] = a;
+  }
+  __syncthreads();
+  if (tid < D) b[tid] = beta * (b[tid] - m * t1[tid]);   // beta Z^T (y - m)
+  int my_info = 0;
+  __syncthreads();
+  for (int q = 0; q < D; ++q) {
+    const double piv = A[q * ld + q];
+    const double lq = sqrt(piv), inv = 1.0 / lq;
+    if (tid == 0 && !(piv > 0.0 && piv < INFINITY) && my_info == 0) my_info = q + 1;
+    __syncthreads();
+    if (tid < D) {
+      if (tid > q) A[tid * ld + q] *= inv;
+      if (tid == q) A[q * ld + q] = lq;
+    }
+    __syncthreads();
+    const int n = D - 1 - q;
+    for (int e = tid; e < n * n; e += blockDim.x) {
+      const int i = q + 1 + e / n, k = q + 1 + e % n;
+      if (k <= i) A[i * ld + k] -= A[i * ld + q] * A[k * ld + q];
+    }
+    __syncthreads();
+  }
+  if (tid >= 32) return;
+  // warp 0: lane l owns rows l and l + 32 of the right-hand side; each step broadcasts the solved entry
+  const int lane = tid;
+  double r0 = lane < D ? b[lane] : 0.0, r1 = lane + 32 < D ? b[lane + 32] : 0.0;
+  for (int i = 0; i < D; ++i) {                                   // u = L_A^-1 b
+    const double own = i < 32 ? r0 : r1;
+    const double ui = __shfl_sync(0xffffffffu, own, i & 31) / A[i * ld + i];
+    if (lane == (i & 31)) { if (i < 32) r0 = ui; else r1 = ui; }
+    if (lane > i && lane < D) r0 -= A[lane * ld + i] * ui;
+    if (lane + 32 > i && lane + 32 < D) r1 -= A[(lane + 32) * ld + i] * ui;
+  }
+  for (int i = D - 1; i >= 0; --i) {                              // w = L_A^-T u
+    const double own = i < 32 ? r0 : r1;
+    const double wi = __shfl_sync(0xffffffffu, own, i & 31) / A[i * ld + i];
+    if (lane == (i & 31)) { if (i < 32) r0 = wi; else r1 = wi; }
+    if (lane < i) r0 -= A[i * ld + lane] * wi;
+    if (lane + 32 < i) r1 -= A[i * ld + lane + 32] * wi;
+  }
+  double ld_sum = (lane < D ? log(A[lane * ld + lane]) : 0.0) + (lane + 32 < D ? log(A[(lane + 32) * ld + lane + 32]) : 0.0);
+  double ww = (lane < D ? r0 * r0 : 0.0) + (lane + 32 < D ? r1 * r1 : 0.0);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    ld_sum += __shfl_xor_sync(0xffffffffu, ld_sum, o);
+    ww += __shfl_xor_sync(0xffffffffu, ww, o);
+  }
+  if (lane < D) w_out[(long long)s * D + lane] = r0;
+  if (lane + 32 < D) w_out[(long long)s * D + lane + 32] = r1;
+  if (lane == 0) {
+    stat[s * 2 + 0] = ld_sum;
+    stat[s * 2 + 1] = ww;
+    info[s] = my_info;
+  }
+}
+
+// res[s][block] = sum over the block's rows of (y_i - m_s - z_i^T w_s)^2.  A fixed row partition (it depends on N only), one warp
+// per row (lane l holds z_il and z_i,l+32), eight draws per pass over the rows, warp sums added in warp order.
+constexpr int kResBlocks = 296;
+constexpr int kResDraws = 8;
+
+__global__ void __launch_bounds__(256)
+blr_residual_kernel(const double* __restrict__ Z, const double* __restrict__ y, int N, int D, const double* __restrict__ w,
+                    const double* __restrict__ par, int S, double* __restrict__ res) {
+  __shared__ double wsum[8][kResDraws];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int rows_per = (N + gridDim.x - 1) / gridDim.x;
+  const int r0 = blockIdx.x * rows_per, r1 = min(N, r0 + rows_per);
+  for (int s0 = 0; s0 < S; s0 += kResDraws) {
+    double wa[kResDraws], wb[kResDraws], m[kResDraws], acc[kResDraws];
+#pragma unroll
+    for (int j = 0; j < kResDraws; ++j) {
+      const bool on = s0 + j < S;
+      wa[j] = on && lane < D ? w[(long long)(s0 + j) * D + lane] : 0.0;
+      wb[j] = on && lane + 32 < D ? w[(long long)(s0 + j) * D + lane + 32] : 0.0;
+      m[j] = on ? par[(s0 + j) * 4 + 2] : 0.0;
+      acc[j] = 0.0;
+    }
+    for (int i = r0 + warp; i < r1; i += 8) {
+      const double za = lane < D ? Z[(long long)i * D + lane] : 0.0;
+      const double zb = lane + 32 < D ? Z[(long long)i * D + lane + 32] : 0.0;
+      const double yi = y[i];
+#pragma unroll
+      for (int j = 0; j < kResDraws; ++j) {
+        double d = fma(zb, wb[j], za * wa[j]);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
+        const double r = (yi - m[j]) - d;
+        acc[j] = fma(r, r, acc[j]);
+      }
+    }
+    if (lane == 0) {
+#pragma unroll
+      for (int j = 0; j < kResDraws; ++j) wsum[warp][j] = acc[j];
+    }
+    __syncthreads();
+    if (threadIdx.x < kResDraws && s0 + (int)threadIdx.x < S) {
+      double a = 0.0;
+      for (int k = 0; k < 8; ++k) a += wsum[k][threadIdx.x];
+      res[(long long)(s0 + threadIdx.x) * gridDim.x + blockIdx.x] = a;
+    }
+    __syncthreads();
+  }
+}
+
+// one thread per draw: the residual partials in block order, then log p(y | row s); -inf for a failed factor or a
+// non-finite value
+__global__ void blr_evidence_finish_kernel(const double* __restrict__ res, int n_blocks, const double* __restrict__ stat,
+                                           const double* __restrict__ hyp, const double* __restrict__ par, const int* __restrict__ info,
+                                           int N, int D, int S, double* __restrict__ logev) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  double e = 0.0;
+  for (int p = 0; p < n_blocks; ++p) e += res[(long long)s * n_blocks + p];
+  const double alpha_p = par[s * 4 + 0], beta = par[s * 4 + 1];
+  const double E = 0.5 * beta * e + 0.5 * alpha_p * stat[s * 2 + 1];
+  const double lp = 0.5 * D * hyp[s * 3 + 0] + 0.5 * N * hyp[s * 3 + 1] - E - stat[s * 2 + 0] - 0.5 * N * 1.83787706640934548356;
+  logev[s] = (info[s] == 0 && isfinite(lp)) ? lp : -INFINITY;
 }
 
 // moments of draws [0, S) for a tile of 128 candidates per block
@@ -441,6 +600,9 @@ void b7_blr_free(b7_blr* blr) {
   b7_pool_free(blr->ctx, blr->Linv);
   b7_pool_free(blr->ctx, blr->w);
   b7_pool_free(blr->ctx, blr->par);
+  for (double* p : {blr->Z, blr->y, blr->partial, blr->gram, blr->hyp, blr->ev_w, blr->ev_stat, blr->ev_res, blr->ev_out})
+    b7_pool_free(blr->ctx, p);
+  b7_pool_free(blr->ctx, blr->ev_info);
   delete blr;
 }
 
@@ -490,7 +652,9 @@ int b7_blr_fit(b7_ctx* ctx, const double* Z0, const double* y, int N, int D, con
   cudaMemcpyAsync(hi.data(), dinfo, S * sizeof(int), cudaMemcpyDeviceToHost, st);
   cudaError_t e = cudaStreamSynchronize(st);
   if (e == cudaSuccess) e = cudaGetLastError();
-  b7_pool_free(ctx, dZ); b7_pool_free(ctx, dy); b7_pool_free(ctx, partial); b7_pool_free(ctx, dinfo);
+  b7_pool_free(ctx, dinfo);
+  // observations and Gram partials stay on the device for b7_blr_refit
+  blr->Z = dZ; blr->y = dy; blr->partial = partial; blr->gram_blocks = blocks;
   if (e != cudaSuccess) { b7_set_error("blr_fit: %s", cudaGetErrorString(e)); b7_blr_free(blr); return B7_ERR_CUDA; }
   int worst = 0;
   for (int s = 0; s < S; ++s) { if (info) info[s] = hi[s]; if (hi[s] && !worst) worst = hi[s]; }
@@ -498,8 +662,72 @@ int b7_blr_fit(b7_ctx* ctx, const double* Z0, const double* y, int N, int D, con
   return worst;   // LAPACK-style: >0 = first failing pivot of the first failing draw
 }
 
+int b7_blr_refit(b7_blr* blr, const double* hyp, int flags, int* info, double* logev) {
+  if (!blr || !hyp || (flags != B7_FIT_PREDICT && flags != B7_FIT_LOGML_ONLY)) {
+    b7_set_error("blr_refit: bad arguments (flags must be B7_FIT_PREDICT or B7_FIT_LOGML_ONLY)");
+    return B7_ERR_ARG;
+  }
+  b7_ctx* ctx = blr->ctx;
+  B7_CUDA(cudaSetDevice(ctx->device));
+  const int N = blr->N, D = blr->D, S = blr->S, n_out = D * D + 2 * D;
+  const int res_blocks = std::min(kResBlocks, (N + 63) / 64);
+  cudaStream_t st = ctx->stream;
+  if (!blr->gram) {
+    B7_CHECK(dalloc(ctx, &blr->gram, (size_t)n_out));
+    B7_CHECK(dalloc(ctx, &blr->hyp, (size_t)S * 3));
+    B7_CHECK(dalloc(ctx, &blr->ev_w, (size_t)S * D));
+    B7_CHECK(dalloc(ctx, &blr->ev_stat, (size_t)S * 2));
+    B7_CHECK(dalloc(ctx, &blr->ev_res, (size_t)S * res_blocks));
+    B7_CHECK(dalloc(ctx, &blr->ev_out, (size_t)S));
+    B7_CHECK(dalloc(ctx, &blr->ev_info, (size_t)2 * S));
+    blr_gram_reduce_kernel<<<(n_out + 255) / 256, 256, 0, st>>>(blr->partial, blr->gram_blocks, n_out, blr->gram);
+    b7_count(ctx);
+  }
+  for (int s = 0; s < S; ++s) {                       // same conversion as b7_blr_fit
+    const double ap = exp(hyp[s * 3 + 0]), be = exp(hyp[s * 3 + 1]);
+    blr->par_host[s * 4 + 0] = ap; blr->par_host[s * 4 + 1] = be; blr->par_host[s * 4 + 2] = hyp[s * 3 + 2];
+    blr->par_host[s * 4 + 3] = 1.0 / be;
+  }
+  cudaMemcpyAsync(blr->par, blr->par_host.data(), (size_t)S * 4 * 8, cudaMemcpyHostToDevice, st);
+  cudaMemcpyAsync(blr->hyp, hyp, (size_t)S * 3 * 8, cudaMemcpyHostToDevice, st);
+  const bool predict = flags == B7_FIT_PREDICT;
+  StageTimer t(ctx, ST_BLR);
+  blr_evidence_kernel<<<S, 256, ((size_t)D * (D + 1) + 2 * D) * 8, st>>>(blr->gram, D, blr->par, blr->ev_w, blr->ev_stat, blr->ev_info);
+  blr_residual_kernel<<<res_blocks, 256, 0, st>>>(blr->Z, blr->y, N, D, blr->ev_w, blr->par, S, blr->ev_res);
+  blr_evidence_finish_kernel<<<(S + 127) / 128, 128, 0, st>>>(blr->ev_res, res_blocks, blr->ev_stat, blr->hyp, blr->par, blr->ev_info, N, D, S,
+                                                              blr->ev_out);
+  // the predictor: the kept partials through blr_finish_kernel, exactly as b7_blr_fit reduces them
+  if (predict)
+    blr_finish_kernel<<<S, 256, (2 * D * (D + 1) + 2 * D) * 8, st>>>(blr->partial, blr->gram_blocks, D, blr->par, blr->Linv, blr->w,
+                                                                      blr->ev_info + S);
+  b7_count(ctx, predict ? 4 : 3);
+  t.stop(predict ? 4 : 3);
+  std::vector<int> hi((size_t)2 * S);
+  std::vector<double> hl((size_t)S);
+  cudaMemcpyAsync(hi.data(), blr->ev_info, (size_t)(predict ? 2 : 1) * S * sizeof(int), cudaMemcpyDeviceToHost, st);
+  cudaMemcpyAsync(hl.data(), blr->ev_out, (size_t)S * 8, cudaMemcpyDeviceToHost, st);
+  cudaError_t e = cudaStreamSynchronize(st);
+  if (e == cudaSuccess) e = cudaGetLastError();
+  if (e != cudaSuccess) { b7_set_error("blr_refit: %s", cudaGetErrorString(e)); blr->ready = false; return B7_ERR_CUDA; }
+  blr->ready = predict;
+  int worst = 0;
+  for (int s = 0; s < S; ++s) {
+    const int f = hi[s] ? hi[s] : (predict ? hi[S + s] : 0);
+    if (info) info[s] = f;
+    if (logev) logev[s] = f ? -INFINITY : hl[s];
+    if (f && !worst) worst = f;
+  }
+  return worst;
+}
+
+int b7_blr_num_draws(b7_blr* blr) {
+  if (!blr) { b7_set_error("blr_num_draws: null handle"); return B7_ERR_ARG; }
+  return blr->S;
+}
+
 int b7_blr_predict(b7_blr* blr, int s, const double* Z1, int64_t M, double* mean, double* var) {
   if (!blr || s < 0 || s >= blr->S || M < 0 || (M > 0 && (!Z1 || !mean || !var))) { b7_set_error("blr_predict: bad arguments"); return B7_ERR_ARG; }
+  if (!blr->ready) { b7_set_error("blr_predict: the last refit was B7_FIT_LOGML_ONLY; refit with B7_FIT_PREDICT first"); return B7_ERR_STATE; }
   b7_ctx* ctx = blr->ctx;
   B7_CUDA(cudaSetDevice(ctx->device));
   const int64_t chunk = 1 << 20;
@@ -532,6 +760,7 @@ static int blr_score_impl(b7_blr* blr, b7_grid* features, int n_layers, const in
     return B7_ERR_ARG;
   }
   if (features->ctx != blr->ctx) { b7_set_error("blr_score: the feature grid and the model live on different contexts / devices"); return B7_ERR_ARG; }
+  if (!blr->ready) { b7_set_error("blr_score: the last refit was B7_FIT_LOGML_ONLY; refit with B7_FIT_PREDICT first"); return B7_ERR_STATE; }
   b7_ctx* ctx = blr->ctx;
   B7_CUDA(cudaSetDevice(ctx->device));
   const int64_t M = features->rows;

@@ -270,11 +270,27 @@ class BLRFactors:
             raise ValueError("BLR hyp rows are [log alpha_p, log beta, m]")
         self.N, self.D = Z0.shape
         self.S = hyp.shape[0]
+        self.hyp = hyp
         self.handle = C.c_void_p()
         info = (C.c_int * self.S)()
         L.check(L.lib().b7_blr_fit(self.ctx.handle, L.dptr(Z0), L.dptr(y), self.N, self.D, L.dptr(hyp), self.S,
                                    C.byref(self.handle), info), "b7_blr_fit")
         self.info = np.array(list(info))
+        self.logev = None
+
+    def refit(self, hyp, flags=L.FIT_PREDICT):
+        """New S x 3 rows on the same features and responses (all device buffers reused) -> (logev, info):
+        log p(y | row) per row (-inf where info != 0).  FIT_LOGML_ONLY leaves the handle unable to predict until the
+        next FIT_PREDICT refit."""
+        hyp = np.atleast_2d(L.as_f64(hyp))
+        if hyp.shape != self.hyp.shape:
+            raise ValueError("refit needs the same S x 3 shape as the original fit")
+        info = (C.c_int * self.S)()
+        self.logev = np.empty(self.S)
+        L.check(L.lib().b7_blr_refit(self.handle, L.dptr(hyp), flags, info, L.dptr(self.logev)), "b7_blr_refit")
+        self.hyp = hyp
+        self.info = np.array(list(info))
+        return self.logev, self.info
 
     def predict(self, s, Z1):
         Z1 = np.atleast_2d(L.as_f64(Z1))
@@ -332,15 +348,31 @@ def dngo_score(blr, grid, weights, biases, relu_last=True, kind=L.SCORE_EI, trad
 
 class bayes_linear:
     """gp.models.bayes_linear as used by models/dngo.lua:77-79,174:
-    predict(Z0, Y0, Z1, nil, hyp, req) with hyp == 'marginalize' or a S x 3 array."""
+    predict(Z0, Y0, Z1, nil, hyp, req) with hyp == 'marginalize' or a S x 3 array.
 
-    def __init__(self, config=None, ctx=None):
+    config keys: alpha_p (1), beta (1e2) -- the fixed row [log alpha_p, log beta, mean(Y0)] that 'marginalize' uses by
+    default; sampler (None; 'slice': 'marginalize' averages over `nSamples` successive states of a slice-sampling chain on
+    log p(y | h) + log p(h), started at the fixed row and kept across calls like gp_regressor.sample_hypers keeps its
+    chain), nSamples (10), prior_std (2), speculative (True), spec_width (8), burnin (0: chain steps discarded when the
+    chain starts).
+    """
+
+    def __init__(self, config=None, ctx=None, rng=None):
         c = dict(config or {})
         c.setdefault("alpha_p", 1.0)
         c.setdefault("beta", 1e2)
+        c.setdefault("sampler", None)
+        c.setdefault("nSamples", 10)
+        c.setdefault("prior_std", 2.0)     # declared: independent N(0, prior_std^2) on every hyp entry, as for the GP
+        c.setdefault("speculative", True)  # batched density evaluations; the chain is identical either way
+        c.setdefault("spec_width", 8)
+        c.setdefault("burnin", 0)
         self.config = c
         self.ctx = ctx
+        self.rng = rng or np.random.default_rng(0)
         self.hyp = None
+        self._density_key = None
+        self._density = None
 
     def class_(self):
         return "gp.models.bayes_linear"
@@ -348,9 +380,72 @@ class bayes_linear:
     def default_hyp(self, Y0):
         return np.array([[math.log(self.config["alpha_p"]), math.log(self.config["beta"]), float(np.mean(Y0))]])
 
+    def _density_handle(self, Z0, Y0, rows, W):
+        """The resident handle of W slots for (Z0, Y0), refitted to `rows` (W x 3) for the log evidence only."""
+        key = (np.asarray(Z0).tobytes(), np.asarray(Y0).tobytes(), W)
+        if self._density_key != key:                 # Z0, y and the Gram partials stay resident across the evaluations
+            if self._density is not None:
+                self._density.free()
+            self._density = BLRFactors(Z0, Y0, rows, self.ctx)
+            self._density_key = key
+        self._density.refit(rows, L.FIT_LOGML_ONLY)
+        return self._density
+
+    def log_density(self, h, Z0, Y0):
+        """log p(y | h) + log p(h): one density evaluation of the slice sampler on a single-slot handle."""
+        h = L.as_f64(h).reshape(1, -1)
+        f = self._density_handle(Z0, Y0, h, 1)
+        lp = float(f.logev[0]) if f.info[0] == 0 and np.isfinite(f.logev[0]) else -np.inf
+        sd = self.config["prior_std"]
+        return lp - 0.5 * float(np.sum((h / sd) ** 2))
+
+    def log_density_batch(self, H, Z0, Y0):
+        """k density evaluations in one device call per `spec_width` rows: what the speculative sampler asks for.
+        The handle keeps `spec_width` slots; short batches repeat their last row."""
+        H = np.atleast_2d(L.as_f64(H))
+        k, W = H.shape[0], max(int(self.config["spec_width"]), 3)
+        out = []
+        for c0 in range(0, k, W):
+            chunk = H[c0:c0 + W]
+            n = chunk.shape[0]
+            padded = np.concatenate([chunk, np.repeat(chunk[-1:], W - n, 0)], 0) if n < W else chunk
+            f = self._density_handle(Z0, Y0, padded, W)
+            sd = self.config["prior_std"]
+            for i in range(n):
+                lp = float(f.logev[i]) if f.info[i] == 0 and np.isfinite(f.logev[i]) else -np.inf
+                out.append(lp - 0.5 * float(np.sum((chunk[i] / sd) ** 2)))
+        return out
+
+    def _step(self, x, Z0, Y0):
+        if self.config["speculative"]:
+            return slice_speculative()(lambda V, a: self.log_density_batch(V, Z0, Y0), x, {"nSamples": 1}, None,
+                                       rng=self.rng, width=int(self.config["spec_width"]))
+        return slice_sampler()(lambda v, a: self.log_density(v, Z0, Y0), x, {"nSamples": 1}, None, rng=self.rng)
+
+    def sample_hypers(self, Z0, Y0, single=False):
+        """Slice-sample the (alpha_p, beta, m) posterior; the chain starts at the fixed row and its state is kept."""
+        Z0 = np.atleast_2d(L.as_f64(Z0))
+        Y0 = L.as_f64(Y0).reshape(-1)
+        if self.hyp is None:
+            x = self.default_hyp(Y0)
+            for _ in range(int(self.config["burnin"])):
+                x = self._step(x, Z0, Y0)
+            self.hyp = x[0].copy()
+        n = 1 if single else int(self.config["nSamples"])
+        out = np.empty((n, self.hyp.size))
+        x = self.hyp.reshape(1, -1).copy()
+        for i in range(n):
+            x = self._step(x, Z0, Y0)
+            out[i] = x[0]
+        self.hyp = out[-1].copy()
+        return out[0] if single else out
+
     def factors(self, Z0, Y0, hyp=None) -> BLRFactors:
         if hyp is None or (isinstance(hyp, str) and hyp == "marginalize"):
-            hyp = self.hyp if self.hyp is not None else self.default_hyp(Y0)
+            if self.config["sampler"] == "slice":
+                hyp = self.sample_hypers(Z0, Y0)
+            else:
+                hyp = self.hyp if self.hyp is not None else self.default_hyp(Y0)
         return BLRFactors(Z0, Y0, hyp, self.ctx)
 
     def predict(self, Z0, Y0, Z1, _unused=None, hyp=None, req=None):
@@ -364,10 +459,10 @@ class dngo:
     """models/dngo.lua BLR head only (SURVEY a-16): `basis` maps X -> features (the trained network of
     the reference, models/dngo.lua:83-105,155-171, is out of scope and is passed in as a callable)."""
 
-    def __init__(self, config=None, basis=None, ctx=None):
+    def __init__(self, config=None, basis=None, ctx=None, rng=None):
         self.config = dict(config or {})
         self.basis = basis
-        self.predictor = bayes_linear(self.config.get("predictor"), ctx)
+        self.predictor = bayes_linear(self.config.get("predictor"), ctx, rng)
 
     def class_(self):
         return "bot7.models.dngo"

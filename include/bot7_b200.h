@@ -154,6 +154,16 @@ int b7_mlp_features(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, con
                     const double* const* b, int relu_last, b7_grid** out);
 int b7_blr_fit(b7_ctx* ctx, const double* Z0, const double* y, int N, int D, const double* hyp, int S,
                b7_blr** out, int* info);
+/* Same features and responses, new S x 3 rows [log alpha_p, log beta, m], every device buffer reused: the density the
+ * slice sampler evaluates for bayes_linear's hyper-parameters (declared arithmetic, DESIGN.md section 4.5):
+ *   log p(y | h) = D/2 log alpha_p + N/2 log beta - E - sum_i log (L_A)_ii - N/2 log 2 pi,
+ *   E = beta/2 |y - m - Z0 w|^2 + alpha_p/2 |w|^2.
+ * flags: B7_FIT_PREDICT (also refresh L_A^-1, w for b7_blr_predict / b7_blr_score / b7_dngo_score, bit-identical to a
+ * b7_blr_fit with the same rows) or B7_FIT_LOGML_ONLY (the handle cannot predict until the next B7_FIT_PREDICT).
+ * logev[s]: log p(y | row s) (-inf when info[s] != 0 or the value is not finite); a row's result does not depend on the
+ * other rows of the call. */
+int b7_blr_refit(b7_blr* blr, const double* hyp, int flags, int* info /* S, nullable */, double* logev /* S, nullable */);
+int b7_blr_num_draws(b7_blr* blr);
 int b7_blr_predict(b7_blr* blr, int s, const double* Z1, int64_t M, double* mean, double* var);
 int b7_blr_score(b7_blr* blr, b7_grid* features, int kind, double tradeoff, int bound, double sign,
                  double fmin, double* score_host, int64_t* argmax, int64_t* argmax_original,

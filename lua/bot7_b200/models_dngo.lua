@@ -6,6 +6,9 @@
 --   * bots.bayesopt (bayesopt.lua) calls model:acquire(...), which fuses basis + head + score + argmax in one pass
 --     over the grid (b7_dngo_score) and never stores Z1.
 -- BLR hyper rows [log alpha_p, log beta, m] follow oracle/SPEC.md (gpTorch7's bayes_linear is not available).
+-- With config.predictor.sampler == 'slice' the rows that 'marginalize' averages over are nSamples successive states of a slice
+-- sampling chain on the BLR log evidence + the N(0, prior_std^2) prior (dngo:sample_blr_hypers, b7_blr_refit on a resident
+-- handle); without it the head uses the one fixed row [log alpha_p, log beta, mean(Y0)], as it always has.
 local B   = require('bot7_b200.ffi')
 local ffi = require('ffi')
 
@@ -62,11 +65,88 @@ function dngo:blr_hyp(Y0, hyp)
   return torch.DoubleTensor{{math.log(p.alpha_p or 1.0), math.log(p.beta or 1e2), Y0:mean()}}
 end
 
+-- settings of the hyper-parameter chain (config.predictor, read with the defaults of the Python twin bayes_linear)
+local function chain_config(self)
+  local p = self.config.predictor or {}
+  return {sampler = p.sampler, nSamples = p.nSamples or 10, prior_std = p.prior_std or 2.0, speculative = p.speculative ~= false,
+          spec_width = math.max(p.spec_width or 8, 1), burnin = p.burnin or 0}
+end
+
 function dngo:blr_fit(Z0, Y0, hyp)
+  if not torch.isTensor(hyp) and chain_config(self).sampler == 'slice' then hyp = self:sample_blr_hypers(Z0, Y0) end
   local Z0, Y0, hyp = Z0:contiguous():double(), Y0:contiguous():double(), self:blr_hyp(Y0, hyp)
   local box, info = ffi.new('b7_blr*[1]'), ffi.new('int[?]', hyp:size(1))
   B.check(B.C.b7_blr_fit(B.context(), Z0:data(), Y0:data(), Z0:size(1), Z0:size(2), hyp:data(), hyp:size(1), box, info), 'b7_blr_fit')
+  self.blr_rows = hyp
   return ffi.gc(box[0], B.C.b7_blr_free), hyp:size(1)
+end
+
+---------------- log p(y | h) + log p(h) of the BLR head for the rows of H: the density the slice sampler evaluates.
+-- Z0 and y stay resident between evaluations (b7_blr_refit on one handle of W slots); a failed factorisation or a
+-- non-finite evidence is -inf, so the sampler rejects the point.
+function dngo:blr_log_density_batch(H, Z0, Y0, W)
+  local c    = chain_config(self)
+  local H    = H:contiguous():double():view(-1, 3)
+  local k    = H:size(1)
+  local W    = W or c.spec_width
+  local out  = torch.DoubleTensor(k)
+  local pad  = torch.DoubleTensor(W, 3)
+  local info, logev = ffi.new('int[?]', W), torch.DoubleTensor(W)
+  self._blr_density = self._blr_density or {}
+  for c0 = 1, k, W do
+    local n = math.min(W, k - c0 + 1)
+    pad:narrow(1, 1, n):copy(H:narrow(1, c0, n))
+    for r = n + 1, W do pad[r]:copy(H[c0 + n - 1]) end       -- short batches repeat their last row
+    local slot = self._blr_density[W]
+    if slot == nil or slot.Z ~= Z0 or slot.Y ~= Y0 then
+      local box, finfo = ffi.new('b7_blr*[1]'), ffi.new('int[?]', W)
+      B.check(B.C.b7_blr_fit(B.context(), Z0:data(), Y0:data(), Z0:size(1), Z0:size(2), pad:data(), W, box, finfo), 'b7_blr_fit')
+      slot = {blr = ffi.gc(box[0], B.C.b7_blr_free), Z = Z0, Y = Y0}
+      self._blr_density[W] = slot
+    end
+    B.check(B.C.b7_blr_refit(slot.blr, pad:data(), B.C.B7_FIT_LOGML_ONLY, info, logev:data()), 'b7_blr_refit')
+    for i = 1, n do
+      local lp = logev[i]
+      if info[i - 1] ~= 0 or lp ~= lp or lp == math.huge or lp == -math.huge then lp = -math.huge end
+      out[c0 + i - 1] = lp - 0.5 * H[c0 + i - 1]:clone():div(c.prior_std):pow(2):sum()
+    end
+  end
+  return out
+end
+
+---------------- the (alpha_p, beta, m) rows 'marginalize' averages over: nSamples successive states of the chain, which starts
+-- at the fixed row of blr_hyp (after `burnin` discarded steps) and is kept across calls, like gp_regressor:sample_hypers.
+-- sampler_spec.lua batches spec_width evaluations per device call; speculative = false uses bot7.samplers.slice.
+function dngo:sample_blr_hypers(Z0, Y0, single)
+  local c = chain_config(self)
+  local Z0, Y0 = Z0:contiguous():double(), Y0:contiguous():double()
+  local sampler, f
+  if c.speculative then
+    sampler = require('bot7_b200.sampler_spec')()
+    f       = function(V, args) return self:blr_log_density_batch(V, Z0, Y0) end
+  else
+    sampler = bot7.samplers.slice()
+    f       = function(x, args) return self:blr_log_density_batch(x, Z0, Y0, 1)[1] end
+  end
+  local function step(x)
+    if c.speculative then return sampler(f, x, {nSamples = 1}, nil, c.spec_width) end
+    return sampler(f, x, {nSamples = 1}, nil)
+  end
+  if self.blr_state == nil then
+    local x = self:blr_hyp(Y0, nil)
+    for _ = 1, c.burnin do x = step(x) end
+    self.blr_state = x:view(1, -1):clone()
+  end
+  local n   = single and 1 or c.nSamples
+  local out = torch.DoubleTensor(n, 3)
+  local x   = self.blr_state:view(1, -1):clone()
+  for i = 1, n do
+    x = step(x)
+    out[i]:copy(x[1])
+  end
+  self.blr_state = out[n]:view(1, -1):clone()
+  if single then return out[1]:view(1, -1) end
+  return out
 end
 
 ---------------- models/dngo.lua:108-175: same signature and return value
