@@ -90,6 +90,9 @@ SIGNATURES = {
     "b7_grid_remove_sharded": (_i, [_p, C.POINTER(_p), _l, _dp]),
     "b7_gp_fit_sharded": (_i, [_p, _i, _dp, _dp, _i, _i, _dp, _i, _i, _i, C.POINTER(_p), _ip, _dp, _dp, _dp]),
     "b7_acq_score_multi": (_i, [_p, C.POINTER(_p), C.POINTER(_p), _i, _d, _i, _d, _d, _dp, _lp, _lp, _dp, _lp]),
+    "b7_blr_fit_multi": (_i, [_p, _dp, _dp, _i, _i, _dp, _i, C.POINTER(_p), _ip]),
+    "b7_dngo_score_multi": (_i, [_p, C.POINTER(_p), C.POINTER(_p), _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _i, _i, _d, _i, _d, _d, _dp,
+                                 _lp, _lp, _dp, _lp]),
 }
 
 

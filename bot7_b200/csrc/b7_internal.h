@@ -140,6 +140,8 @@ struct b7_blr {
 // sharded fit (multi.cu): before / after the exchange of the per-draw state (api.cu)
 int b7_gp_prepare_gather(b7_gp* gp, int s0, int count);
 int b7_gp_finish_gather(b7_gp* gp, bool slices_exchanged);
+// whether b7_dngo_score can run a basis of these widths (dims[0 .. n_layers]) in front of a head of width D (blr_dmma.cu)
+bool b7_dngo_tiles_fit(int n_layers, const int* dims, int D);
 
 // stream-ordered pool allocation on the context stream (api.cu)
 int b7_pool_alloc(b7_ctx* ctx, void** p, size_t bytes);

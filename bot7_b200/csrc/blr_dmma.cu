@@ -306,17 +306,10 @@ dngo_tile_kernel(const double* __restrict__ in, long long M, Plan pl, Ptrs pt, c
   }
 }
 
-}  // namespace
-
-// Plans the shared memory, uploads nothing (all pointers are device pointers) and launches.  Returns 1 if the shapes
-// do not fit the tile kernel (the caller then uses the per-candidate kernels of blr.cu).
-int b7_launch_dngo_tiles(b7_ctx* ctx, const double* in, int64_t M, int n_layers, const int* dims, const double* const* W_dev,
-                         const double* const* b_dev, int relu_last, const double* Linv, const double* w, const double* par, int D, int S,
-                         int64_t ld_out, double* mean, double* var, double* feat_out) {
-  if (M <= 0) return 0;
+// Plans the shared memory of one launch; returns 1 if the shapes do not fit the tile kernel.
+int plan_tiles(int n_layers, const int* dims, int relu_last, int D, int S, Plan* plan, size_t* smem_bytes) {
   if (n_layers > MAXL) return 1;
   Plan pl = {};
-  Ptrs pt = {};
   pl.n_layers = n_layers;
   pl.S = S;
   int off = 0, wmax = dims[0];
@@ -331,8 +324,6 @@ int b7_launch_dngo_tiles(b7_ctx* ctx, const double* in, int64_t M, int n_layers,
     pl.relu[l] = (l < n_layers - 1 || relu_last) ? 1 : 0;
     pl.w_off[l] = off; off += rows * ld_of(dims[l]);
     pl.b_off[l] = off; off += rows;
-    pt.W[l] = W_dev[l];
-    pt.b[l] = b_dev[l];
   }
   pl.head_rows = S > 0 ? (D + 1 + 7) / 8 * 8 : 0;
   pl.head_off = off; off += S * pl.head_rows * (S > 0 ? ld_of(D) : 0);
@@ -344,6 +335,35 @@ int b7_launch_dngo_tiles(b7_ctx* ctx, const double* in, int64_t M, int n_layers,
   pl.bar_off = off; off += 2;
   const size_t smem = (size_t)off * sizeof(double);
   if (smem > 226 * 1024) return 1;
+  *plan = pl;
+  *smem_bytes = smem;
+  return 0;
+}
+
+}  // namespace
+
+// b7_dngo_score runs its head in chunks of at most four draws and halves the chunk down to one when a launch does not fit:
+// the shapes are usable iff a one-draw launch fits.
+bool b7_dngo_tiles_fit(int n_layers, const int* dims, int D) {
+  Plan pl;
+  size_t smem;
+  return n_layers >= 1 && plan_tiles(n_layers, dims, 0, D, 1, &pl, &smem) == 0;
+}
+
+// Plans the shared memory, uploads nothing (all pointers are device pointers) and launches.  Returns 1 if the shapes
+// do not fit the tile kernel (the caller then uses the per-candidate kernels of blr.cu).
+int b7_launch_dngo_tiles(b7_ctx* ctx, const double* in, int64_t M, int n_layers, const int* dims, const double* const* W_dev,
+                         const double* const* b_dev, int relu_last, const double* Linv, const double* w, const double* par, int D, int S,
+                         int64_t ld_out, double* mean, double* var, double* feat_out) {
+  if (M <= 0) return 0;
+  Plan pl;
+  size_t smem;
+  if (plan_tiles(n_layers, dims, relu_last, D, S, &pl, &smem)) return 1;
+  Ptrs pt = {};
+  for (int l = 0; l < n_layers; ++l) {
+    pt.W[l] = W_dev[l];
+    pt.b[l] = b_dev[l];
+  }
   static bool done[16] = {false};
   if (!done[ctx->device & 15]) {
     B7_CUDA(cudaFuncSetAttribute(dngo_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));

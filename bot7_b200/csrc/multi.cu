@@ -91,7 +91,7 @@ struct b7_comm {
   bool owns_ctx = true;
   std::vector<b7_ctx*> ctx;          // one per local device
   std::vector<ncclComm_t> nccl;      // one per local device (empty when world == 1)
-  std::vector<double*> triple;       // per local device: world x 3 doubles (best, index, nan) for the combine
+  std::vector<double*> triple;       // per local device: world x 4 words for the exchanges of the combine (see exchange_status)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // exchange timing on the first local device (the context's own timer events
                                               // belong to the caller's b7_timer_begin / b7_timer_end)
   int n_local() const { return (int)ctx.size(); }
@@ -149,7 +149,7 @@ int comm_finish_init(b7_comm* c) {
   for (int i = 0; i < c->n_local(); ++i) {
     B7_CUDA(cudaSetDevice(c->ctx[i]->device));
     double* t = nullptr;
-    B7_CHECK(b7_pool_alloc(c->ctx[i], (void**)&t, sizeof(double) * 3 * (size_t)c->world));
+    B7_CHECK(b7_pool_alloc(c->ctx[i], (void**)&t, sizeof(double) * 4 * (size_t)c->world));
     c->triple.push_back(t);
   }
   B7_CUDA(cudaSetDevice(c->ctx[0]->device));
@@ -405,6 +405,55 @@ int b7_gp_fit_sharded(b7_comm* c, int kernel, const double* X, const double* y, 
 
 /* ------------------------------------------------------------------ sharded acquisition */
 
+// The per-rank triples (best score, global original row 1-based or 0, nan count) -> the result every rank reports: larger
+// score, then smaller global original row (the reference's first-maximum scan, bots/bayesopt.lua:96); the compacted index
+// comes from the tombstone list of the whole grid, which every shard holds.
+static void combine_triples(const std::vector<double>& ab, const std::vector<int64_t>& ai, const std::vector<int64_t>& an,
+                            const b7_grid* g, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count) {
+  double bv = NAN;
+  int64_t bi = 0, nn = 0;
+  for (size_t r = 0; r < ab.size(); ++r) {
+    nn += an[r];
+    if (ai[r] <= 0 || ab[r] != ab[r]) continue;
+    if (bi == 0 || ab[r] > bv || (ab[r] == bv && ai[r] < bi)) { bv = ab[r]; bi = ai[r]; }
+  }
+  if (best) *best = bv;
+  if (nan_count) *nan_count = nn;
+  if (argmax_original) *argmax_original = bi;
+  if (argmax) {
+    if (bi <= 0) *argmax = 0;
+    else {
+      const std::vector<int64_t>& rem = g->removed_global;
+      *argmax = bi - (int64_t)(std::lower_bound(rem.begin(), rem.end(), bi - 1) - rem.begin());
+    }
+  }
+}
+
+// One process per GPU: every rank, whether its local step failed or not, enters this one all-gather of its status and the
+// words `mine[0 .. k)` (k <= 3; doubles travel as their exact bit patterns), so that a rank-local failure cannot leave the
+// other ranks waiting inside a collective (a rank whose CUDA context is lost cannot reach it: that case stays fatal, as in
+// b7_gp_fit_sharded's phase-1 exchange).  On success `all` holds world x (1 + k) words.  If a rank failed, that rank
+// returns its own code and message, every other rank B7_ERR_STATE naming the first failed rank.
+static int exchange_status(b7_comm* c, int rc, const int64_t* mine, int k, std::vector<int64_t>& all, const char* what) {
+  b7_ctx* x = c->ctx[0];
+  const int w = 1 + k;
+  const std::string my_msg = rc < 0 ? b7_last_error() : "";
+  int64_t h[4] = {rc < 0 ? rc : 0, 0, 0, 0};
+  for (int j = 0; j < k; ++j) h[1 + j] = mine[j];
+  all.assign((size_t)w * c->world, 0);
+  int64_t* buf = (int64_t*)c->triple[0];
+  cudaError_t e = cudaSetDevice(x->device);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(buf + (size_t)w * c->rank0, h, w * sizeof(int64_t), cudaMemcpyHostToDevice, x->stream);
+  ncclResult_t r = e == cudaSuccess ? g_nccl.AllGather(buf + (size_t)w * c->rank0, buf, w, ncclInt64, c->nccl[0], x->stream) : 1;
+  if (r == 0) e = cudaMemcpyAsync(all.data(), buf, all.size() * sizeof(int64_t), cudaMemcpyDeviceToHost, x->stream);
+  if (r == 0 && e == cudaSuccess) e = cudaStreamSynchronize(x->stream);
+  if (r != 0 || e != cudaSuccess) { b7_set_error("%s: status exchange failed", what); return B7_ERR_NCCL; }
+  if (rc < 0) { b7_set_error("%s", my_msg.c_str()); return rc; }
+  for (int q = 0; q < c->world; ++q)
+    if (all[(size_t)w * q] != 0) { b7_set_error("%s: rank %d failed in its local step", what, q); return B7_ERR_STATE; }
+  return 0;
+}
+
 int b7_acq_score_multi(b7_comm* c, b7_gp** gps, b7_grid** grids, int kind, double tradeoff, int bound, double sign, double fmin,
                        double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count) {
   if (!c || !gps || !grids) { b7_set_error("acq_score_multi: null arguments"); return B7_ERR_ARG; }
@@ -425,7 +474,6 @@ int b7_acq_score_multi(b7_comm* c, b7_gp** gps, b7_grid** grids, int kind, doubl
     return rc_;
   });
   if (rc < 0) return rc;
-  // combine: larger score, then smaller global index (the reference's first-maximum scan, bots/bayesopt.lua:96)
   std::vector<double> ab((size_t)c->world, NAN);
   std::vector<int64_t> ai((size_t)c->world, 0), an((size_t)c->world, 0);
   if (c->world == n) {
@@ -449,23 +497,97 @@ int b7_acq_score_multi(b7_comm* c, b7_gp** gps, b7_grid** grids, int kind, doubl
       memcpy(&an[r], &all[3 * r + 2], 8);
     }
   }
-  double bv = NAN;
-  int64_t bi = 0, nn = 0;
-  for (int r = 0; r < c->world; ++r) {
-    nn += an[r];
-    if (ai[r] <= 0 || ab[r] != ab[r]) continue;
-    if (bi == 0 || ab[r] > bv || (ab[r] == bv && ai[r] < bi)) { bv = ab[r]; bi = ai[r]; }
+  combine_triples(ab, ai, an, grids[0], argmax, argmax_original, best, nan_count);
+  return 0;
+}
+
+/* ------------------------------------------------------------------ DNGO over the communicator */
+
+int b7_blr_fit_multi(b7_comm* c, const double* Z0, const double* y, int N, int D, const double* hyp, int S, b7_blr** out, int* info) {
+  if (!c || !out || S < 1) { b7_set_error("blr_fit_multi: bad arguments (null comm/out or S=%d)", S); return B7_ERR_ARG; }
+  const int n = c->n_local();
+  for (int i = 0; i < n; ++i) out[i] = nullptr;
+  if (c->world == 1) return b7_blr_fit(c->ctx[0], Z0, y, N, D, hyp, S, &out[0], info);
+  // the head is fitted on every device rather than broadcast: the fit has no atomics, so every device holds the same bits
+  std::vector<std::vector<int>> inf((size_t)n, std::vector<int>((size_t)S, 0));
+  std::vector<int> worst((size_t)n, 0);
+  int rc = for_each_local(c, [&](int i) {
+    worst[i] = b7_blr_fit(c->ctx[i], Z0, y, N, D, hyp, S, &out[i], inf[i].data());
+    return worst[i];
+  });
+  if (c->world > n) {
+    std::vector<int64_t> all;
+    rc = exchange_status(c, rc, nullptr, 0, all, "blr_fit_multi");
   }
-  if (best) *best = bv;
-  if (nan_count) *nan_count = nn;
-  if (argmax_original) *argmax_original = bi;
-  if (argmax) {
-    if (bi <= 0) *argmax = 0;
-    else {
-      const std::vector<int64_t>& rem = grids[0]->removed_global;
-      *argmax = bi - (int64_t)(std::lower_bound(rem.begin(), rem.end(), bi - 1) - rem.begin());
+  if (rc < 0) {
+    for (int i = 0; i < n; ++i) { b7_blr_free(out[i]); out[i] = nullptr; }
+    return rc;
+  }
+  if (info)
+    for (int s = 0; s < S; ++s) info[s] = inf[0][s];
+  return worst[0];
+}
+
+int b7_dngo_score_multi(b7_comm* c, b7_blr** blrs, b7_grid** grids, int n_layers, const int* dims, const double* const* W,
+                        const double* const* b, int relu_last, int kind, double tradeoff, int bound, double sign, double fmin,
+                        double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count) {
+  if (!c || !blrs || !grids || n_layers < 1 || !dims || !W || !b || (kind != B7_SCORE_EI && kind != B7_SCORE_CB)) {
+    b7_set_error("dngo_score_multi: bad arguments");
+    return B7_ERR_ARG;
+  }
+  const int n = c->n_local();
+  for (int i = 0; i < n; ++i) {
+    if (!blrs[i] || !grids[i] || blrs[i]->ctx != c->ctx[i] || grids[i]->ctx != c->ctx[i]) {
+      b7_set_error("dngo_score_multi: handle %d does not belong to local device %d of the communicator", i, i);
+      return B7_ERR_ARG;
+    }
+    if (dims[0] != grids[i]->d || dims[n_layers] != blrs[i]->D) {
+      b7_set_error("dngo_score_multi: dims[0] = %d must equal the grid's dims (%d), dims[%d] = %d the head's D (%d)", dims[0], grids[i]->d,
+                   n_layers, dims[n_layers], blrs[i]->D);
+      return B7_ERR_ARG;
+    }
+    if (!blrs[i]->ready) {
+      b7_set_error("dngo_score_multi: the last refit of handle %d was B7_FIT_LOGML_ONLY; refit with B7_FIT_PREDICT first", i);
+      return B7_ERR_STATE;
     }
   }
+  // an empty shard launches nothing and would not notice: check the shapes here, for every rank alike
+  if (!b7_dngo_tiles_fit(n_layers, dims, dims[n_layers])) {
+    b7_set_error("dngo_score: layer shapes do not fit the tile kernel (widths <= 63, at most 4 layers)");
+    return B7_ERR_ARG;
+  }
+  if (c->world == 1)
+    return b7_dngo_score(blrs[0], grids[0], n_layers, dims, W, b, relu_last, kind, tradeoff, bound, sign, fmin, score_host, argmax,
+                         argmax_original, best, nan_count);
+  std::vector<double> tb((size_t)n, NAN);
+  std::vector<int64_t> ti((size_t)n, 0), tn((size_t)n, 0), off((size_t)n, 0);
+  for (int i = 1; i < n; ++i) off[i] = off[i - 1] + grids[i - 1]->rows;
+  int rc = for_each_local(c, [&](int i) {
+    int64_t o = 0;
+    int rc_ = b7_dngo_score(blrs[i], grids[i], n_layers, dims, W, b, relu_last, kind, tradeoff, bound, sign, fmin,
+                            score_host ? score_host + off[i] : nullptr, nullptr, &o, &tb[i], &tn[i]);
+    ti[i] = o > 0 ? o + grids[i]->row_base : 0;      // local original row + the shard's first row: global, 1-based
+    return rc_;
+  });
+  std::vector<double> ab((size_t)c->world, NAN);
+  std::vector<int64_t> ai((size_t)c->world, 0), an((size_t)c->world, 0);
+  if (c->world == n) {
+    if (rc < 0) return rc;
+    for (int i = 0; i < n; ++i) { ab[i] = tb[i]; ai[i] = ti[i]; an[i] = tn[i]; }
+  } else {
+    int64_t mine[3];
+    memcpy(&mine[0], &tb[0], 8);
+    mine[1] = ti[0];
+    mine[2] = tn[0];
+    std::vector<int64_t> all;
+    if ((rc = exchange_status(c, rc, mine, 3, all, "dngo_score_multi")) < 0) return rc;
+    for (int r = 0; r < c->world; ++r) {
+      memcpy(&ab[r], &all[4 * (size_t)r + 1], 8);
+      ai[r] = all[4 * (size_t)r + 2];
+      an[r] = all[4 * (size_t)r + 3];
+    }
+  }
+  combine_triples(ab, ai, an, grids[0], argmax, argmax_original, best, nan_count);
   return 0;
 }
 

@@ -99,7 +99,8 @@ def allgather_factors(factors, S, world, rank, group=None):
 
 
 class Comm:
-    """The multi-GPU block of the C ABI (include/bot7_b200.h): b7_comm_* / b7_gp_fit_sharded / b7_acq_score_multi.
+    """The multi-GPU block of the C ABI (include/bot7_b200.h): b7_comm_* / b7_gp_fit_sharded / b7_acq_score_multi, and for DNGO
+    b7_blr_fit_multi / b7_dngo_score_multi.
 
     Comm.all(n)            one process driving n devices (ncclCommInitAll) -- what the LuaJIT glue does with config.bot.nGPU;
     Comm.from_env()        one process per GPU under torchrun: rank 0 makes the NCCL unique id, torch.distributed carries its
@@ -197,6 +198,41 @@ class Comm:
         am, amo, best, nn = C.c_int64(), C.c_int64(), C.c_double(), C.c_int64()
         L.check(L.lib().b7_acq_score_multi(self.handle, (C.c_void_p * self.n_local)(*gps), self._handles(grids), kind, tradeoff, bound, sign,
                                            fmin, L.dptr(sc), C.byref(am), C.byref(amo), C.byref(best), C.byref(nn)), "b7_acq_score_multi")
+        return best.value, am.value, amo.value, nn.value, sc
+
+    def blr_fit(self, Z0, y, hyp):
+        """b7_blr_fit_multi -> (list of per-device BLR head handles, each holding all S rows, info)."""
+        L = self._L
+        Z0, y = np.atleast_2d(L.as_f64(Z0)), L.as_f64(y).reshape(-1)
+        hyp = np.atleast_2d(L.as_f64(hyp))
+        S = hyp.shape[0]
+        out = (C.c_void_p * self.n_local)()
+        info = (C.c_int * S)()
+        L.check(L.lib().b7_blr_fit_multi(self.handle, L.dptr(Z0), L.dptr(y), Z0.shape[0], Z0.shape[1], L.dptr(hyp), S, out, info),
+                "b7_blr_fit_multi")
+        return [C.c_void_p(out[i]) for i in range(self.n_local)], np.array(list(info))
+
+    def free_blr(self, blrs):
+        for h in blrs:
+            self._L.lib().b7_blr_free(h)
+
+    def dngo_score(self, blrs, grids, weights, biases, relu_last=True, kind=0, tradeoff=0.0, bound=0, sign=-1.0, fmin=0.0,
+                   want_scores=False):
+        """b7_dngo_score_multi -> (best, argmax (global, compacted), argmax_original, nan_count, scores of the local shards or None).
+        weights[l]: (h_out x h_in) like torch nn.Linear.weight; biases[l]: (h_out,)."""
+        L = self._L
+        Ws = [L.as_f64(w) for w in weights]
+        bs = [L.as_f64(b).reshape(-1) for b in biases]
+        n = len(Ws)
+        dims = (C.c_int * (n + 1))(*([Ws[0].shape[1]] + [w.shape[0] for w in Ws]))
+        Wp = (C.POINTER(C.c_double) * n)(*[L.dptr(w) for w in Ws])
+        bp = (C.POINTER(C.c_double) * n)(*[L.dptr(b) for b in bs])
+        rows = sum(int(L.lib().b7_grid_rows(g.handle)) for g in grids)
+        sc = np.empty(rows) if want_scores else None
+        am, amo, best, nn = C.c_int64(), C.c_int64(), C.c_double(), C.c_int64()
+        L.check(L.lib().b7_dngo_score_multi(self.handle, (C.c_void_p * self.n_local)(*blrs), self._handles(grids), n, dims, Wp, bp,
+                                            int(bool(relu_last)), kind, tradeoff, bound, sign, fmin, L.dptr(sc), C.byref(am), C.byref(amo),
+                                            C.byref(best), C.byref(nn)), "b7_dngo_score_multi")
         return best.value, am.value, amo.value, nn.value, sc
 
     def close(self):

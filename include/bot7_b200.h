@@ -218,6 +218,21 @@ int  b7_gp_fit_sharded(b7_comm* comm, int kernel, const double* X, const double*
 int  b7_acq_score_multi(b7_comm* comm, b7_gp** gps, b7_grid** grids, int kind, double tradeoff, int bound, double sign,
                         double fmin, double* score_host, int64_t* argmax, int64_t* argmax_original, double* best,
                         int64_t* nan_count);
+/* DNGO over the communicator (models/dngo.lua:155-174 under bots/bayesopt.lua:65-66 with config.bot.nGPU > 1).  With one
+ * process per GPU every rank enters exactly one all-gather per call, also after its local step failed; then that rank
+ * returns its own error and every other rank B7_ERR_STATE naming it.  With world == 1 both are the one-device calls. */
+/* b7_blr_fit on every local device of the communicator: each handle holds all S rows and predicts / scores bit for bit like a
+ * one-device b7_blr_fit with the same arguments.  out_blrs: n_local handles (free each with b7_blr_free); info: S entries. */
+int  b7_blr_fit_multi(b7_comm* comm, const double* Z0, const double* y, int N, int D, const double* hyp, int S,
+                      b7_blr** out_blrs, int* info /* S, nullable */);
+/* b7_dngo_score over the communicator: each local device runs the fused basis + BLR head + score pass on its shard of the
+ * candidate grid, then the per-rank triples are combined with the rule of b7_acq_score_multi.  Arguments and outputs as
+ * b7_dngo_score and b7_acq_score_multi (score_host: the local shards concatenated in local-device order).  Every handle is
+ * checked before any device work: B7_ERR_ARG for a handle of another device, dims that do not match the grid and the head,
+ * or widths the tile kernel cannot take; B7_ERR_STATE for a head whose last refit was B7_FIT_LOGML_ONLY. */
+int  b7_dngo_score_multi(b7_comm* comm, b7_blr** blrs, b7_grid** grids, int n_layers, const int* dims, const double* const* W,
+                         const double* const* b, int relu_last, int kind, double tradeoff, int bound, double sign, double fmin,
+                         double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count);
 
 #ifdef __cplusplus
 }

@@ -3,6 +3,8 @@
 -- config.bot.nGPU > 1 spreads the same work over the GPUs of the box through the multi-GPU block of the C ABI
 -- (b7_comm_init_all, b7_gp_fit_sharded, b7_acq_score_multi): candidate shards per device, the S factorisations split
 -- over the devices and exchanged once per fit with NCCL, the per-device (best, index) triples combined in the library.
+-- A DNGO model does the same through dngo:acquire_multi (b7_blr_fit_multi: the small BLR head is fitted on every device;
+-- b7_dngo_score_multi: basis + head + score on each shard, same combine).
 local B   = require('bot7_b200.ffi')
 local ffi = require('ffi')
 
@@ -57,7 +59,11 @@ function bot:nominate(candidates)
   local argmax, orig = ffi.new('int64_t[1]'), ffi.new('int64_t[1]')
   local best, nans   = ffi.new('double[1]'), ffi.new('int64_t[1]')
   if self.model:class() == 'bot7.models.dngo' then             -- :65-66
-    argmax[0] = self.model:acquire(X_obs, Y_obs, self.grid_dev, kind, tradeoff, bound, sign)
+    if self.nGPU > 1 then
+      argmax[0] = self.model:acquire_multi(X_obs, Y_obs, self.comm, self.grids, self.nGPU, kind, tradeoff, bound, sign)
+    else
+      argmax[0] = self.model:acquire(X_obs, Y_obs, self.grid_dev, kind, tradeoff, bound, sign)
+    end
   else
     local nSamples = self.config.bot.nSamples
     self.model:sample_hypers(X_obs, Y_obs)                      -- :68 priming draw (result unused)

@@ -4,7 +4,8 @@
 --   * the Linear / ReLU stack below the basis layer is read out of self.network and applied to the device grid by
 --     b7_mlp_features (no 32-row minibatch loop, no host copy of Z1), the head is b7_blr_fit + b7_blr_predict;
 --   * bots.bayesopt (bayesopt.lua) calls model:acquire(...), which fuses basis + head + score + argmax in one pass
---     over the grid (b7_dngo_score) and never stores Z1.
+--     over the grid (b7_dngo_score) and never stores Z1; with config.bot.nGPU > 1 it calls model:acquire_multi(...), the
+--     same pass over the grid's shards (b7_blr_fit_multi + b7_dngo_score_multi).
 -- BLR hyper rows [log alpha_p, log beta, m] follow oracle/SPEC.md (gpTorch7's bayes_linear is not available).
 -- With config.predictor.sampler == 'slice' the rows that 'marginalize' averages over are nSamples successive states of a slice
 -- sampling chain on the BLR log evidence + the N(0, prior_std^2) prior (dngo:sample_blr_hypers, b7_blr_refit on a resident
@@ -72,9 +73,16 @@ local function chain_config(self)
           spec_width = math.max(p.spec_width or 8, 1), burnin = p.burnin or 0}
 end
 
-function dngo:blr_fit(Z0, Y0, hyp)
+-- the S x 3 rows the head is fitted with: `hyp` if given, else the chain's next nSamples states (sampler = 'slice', evaluated
+-- on B.context() also when the head is fitted on several devices) or the one fixed row
+function dngo:blr_rows_for(Z0, Y0, hyp)
   if not torch.isTensor(hyp) and chain_config(self).sampler == 'slice' then hyp = self:sample_blr_hypers(Z0, Y0) end
-  local Z0, Y0, hyp = Z0:contiguous():double(), Y0:contiguous():double(), self:blr_hyp(Y0, hyp)
+  return self:blr_hyp(Y0, hyp)
+end
+
+function dngo:blr_fit(Z0, Y0, hyp)
+  local hyp    = self:blr_rows_for(Z0, Y0, hyp)
+  local Z0, Y0 = Z0:contiguous():double(), Y0:contiguous():double()
   local box, info = ffi.new('b7_blr*[1]'), ffi.new('int[?]', hyp:size(1))
   B.check(B.C.b7_blr_fit(B.context(), Z0:data(), Y0:data(), Z0:size(1), Z0:size(2), hyp:data(), hyp:size(1), box, info), 'b7_blr_fit')
   self.blr_rows = hyp
@@ -183,6 +191,27 @@ function dngo:acquire(X0, Y0, grid_dev, kind, tradeoff, bound, sign, skip)
   local best, nans   = ffi.new('double[1]'), ffi.new('int64_t[1]')
   B.check(B.C.b7_dngo_score(blr, grid_dev, st.n, st.dims, st.W, st.b, st.relu_last, kind, tradeoff, bound, sign, Y0:min(),
                             nil, argmax, orig, best, nans), 'b7_dngo_score')
+  return tonumber(argmax[0]), best[0], tonumber(nans[0])
+end
+
+---------------- the same over the nGPU devices of a communicator (bots.bayesopt with config.bot.nGPU > 1): the head is fitted on
+-- every device (b7_blr_fit_multi), each device scores its shard of the grid and the library combines the argmax
+-- (b7_dngo_score_multi); the result equals acquire's on one device over the whole grid
+function dngo:acquire_multi(X0, Y0, comm, grids, nGPU, kind, tradeoff, bound, sign, skip)
+  if not skip then parent.update_network(self, X0, Y0) end
+  local Z0   = self:host_basis(X0)
+  local hyp  = self:blr_rows_for(Z0, Y0, nil)
+  local Yc   = Y0:contiguous():double()
+  local blrs = ffi.new('b7_blr*[?]', nGPU)
+  B.check(B.C.b7_blr_fit_multi(comm, Z0:data(), Yc:data(), Z0:size(1), Z0:size(2), hyp:data(), hyp:size(1), blrs, nil), 'b7_blr_fit_multi')
+  self.blr_rows = hyp
+  local st = self:basis_stack()
+  local argmax, orig = ffi.new('int64_t[1]'), ffi.new('int64_t[1]')
+  local best, nans   = ffi.new('double[1]'), ffi.new('int64_t[1]')
+  local rc = B.C.b7_dngo_score_multi(comm, blrs, grids, st.n, st.dims, st.W, st.b, st.relu_last, kind, tradeoff, bound, sign, Y0:min(),
+                                     nil, argmax, orig, best, nans)
+  for g = 0, nGPU - 1 do B.C.b7_blr_free(blrs[g]) end
+  B.check(rc, 'b7_dngo_score_multi')
   return tonumber(argmax[0]), best[0], tonumber(nans[0])
 end
 
