@@ -18,6 +18,7 @@ KERNEL_ARDSE, KERNEL_MATERN52 = 0, 1
 SCORE_EI, SCORE_CB = 0, 1
 BOUND_LOWER, BOUND_UPPER = 0, 1
 FIT_PREDICT, FIT_LOGML_ONLY, FIT_DEFER = 0, 1, 2
+ACT_NONE, ACT_RELU, ACT_TANH = 0, 1, 2
 PATH_FP64_DMMA, PATH_INT8_OZAKI = 0, 1
 STAGES = ("sobol", "kbuild", "potrf", "trtri", "kstar", "posterior", "score", "blr")
 
@@ -69,12 +70,14 @@ SIGNATURES = {
     "b7_acq_score_range": (_i, [_p, _p, _l, _l, _i, _d, _i, _d, _d, _dp, _lp, _dp, _lp]),
     "b7_score_moments": (_i, [_p, _i, _dp, _dp, _i, _l, _d, _i, _d, _d, _dp, _lp, _dp, _lp]),
     "b7_mlp_features": (_i, [_p, _p, _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _i, C.POINTER(_p)]),
+    "b7_mlp_features_act": (_i, [_p, _p, _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _ip, C.POINTER(_p)]),
     "b7_blr_fit": (_i, [_p, _dp, _dp, _i, _i, _dp, _i, C.POINTER(_p), _ip]),
     "b7_blr_refit": (_i, [_p, _dp, _i, _ip, _dp]),
     "b7_blr_num_draws": (_i, [_p]),
     "b7_blr_predict": (_i, [_p, _i, _dp, _l, _dp, _dp]),
     "b7_blr_score": (_i, [_p, _p, _i, _d, _i, _d, _d, _dp, _lp, _lp, _dp, _lp]),
     "b7_dngo_score": (_i, [_p, _p, _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _i, _i, _d, _i, _d, _d, _dp, _lp, _lp, _dp, _lp]),
+    "b7_dngo_score_act": (_i, [_p, _p, _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _ip, _i, _d, _i, _d, _d, _dp, _lp, _lp, _dp, _lp]),
     "b7_blr_free": (None, [_p]),
     "b7_comm_init_all": (_i, [_i, _ip, C.POINTER(_p)]),
     "b7_comm_unique_id": (_i, [C.c_char_p]),
@@ -93,6 +96,8 @@ SIGNATURES = {
     "b7_blr_fit_multi": (_i, [_p, _dp, _dp, _i, _i, _dp, _i, C.POINTER(_p), _ip]),
     "b7_dngo_score_multi": (_i, [_p, C.POINTER(_p), C.POINTER(_p), _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _i, _i, _d, _i, _d, _d, _dp,
                                  _lp, _lp, _dp, _lp]),
+    "b7_dngo_score_multi_act": (_i, [_p, C.POINTER(_p), C.POINTER(_p), _i, _ip, C.POINTER(_dp), C.POINTER(_dp), _ip, _i, _d, _i, _d, _d,
+                                     _dp, _lp, _lp, _dp, _lp]),
 }
 
 

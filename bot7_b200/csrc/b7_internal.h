@@ -142,6 +142,15 @@ int b7_gp_prepare_gather(b7_gp* gp, int s0, int count);
 int b7_gp_finish_gather(b7_gp* gp, bool slices_exchanged);
 // whether b7_dngo_score can run a basis of these widths (dims[0 .. n_layers]) in front of a head of width D (blr_dmma.cu)
 bool b7_dngo_tiles_fit(int n_layers, const int* dims, int D);
+// B7_ERR_ARG (message prefixed by `what`) unless act holds n_layers known B7_ACT_* codes (blr.cu)
+int b7_check_act(const char* what, int n_layers, const int* act);
+// the codes of the relu_last form of b7_mlp_features / b7_dngo_score(_multi): ReLU after every layer but the last, after the
+// last one iff relu_last
+inline std::vector<int> b7_relu_codes(int n_layers, int relu_last) {
+  std::vector<int> act((size_t)(n_layers > 0 ? n_layers : 1), B7_ACT_RELU);
+  if (n_layers > 0 && !relu_last) act[(size_t)n_layers - 1] = B7_ACT_NONE;
+  return act;
+}
 
 // stream-ordered pool allocation on the context stream (api.cu)
 int b7_pool_alloc(b7_ctx* ctx, void** p, size_t bytes);

@@ -28,7 +28,7 @@
 int b7_score_grid_size(b7_ctx* ctx, int64_t M);
 // blr_dmma.cu: MLP basis + BLR head on DMMA tiles; returns 1 when the shapes do not fit (use the kernels below)
 int b7_launch_dngo_tiles(b7_ctx* ctx, const double* in, int64_t M, int n_layers, const int* dims, const double* const* W_dev,
-                         const double* const* b_dev, int relu_last, const double* Linv, const double* w, const double* par, int D, int S,
+                         const double* const* b_dev, const int* act, const double* Linv, const double* w, const double* par, int D, int S,
                          int64_t ld_out, double* mean, double* var, double* feat_out);
 
 namespace {
@@ -403,15 +403,15 @@ int launch_moments(b7_ctx* ctx, const double* Z, int64_t M, const b7_blr* blr, i
   }
 }
 
-// ---- DNGO basis: X -> features through the trained ReLU MLP (models/dngo.lua:155-171) ------------------
+// ---- DNGO basis: X -> features through the trained MLP (models/dngo.lua:155-171) ---------------------------
 // One dense layer: out[c][j] = act(b[j] + sum_k W[j][k] in[c][k]).  One thread per candidate keeps its input row in
 // registers (width rounded up to a multiple of 8, <= 64); the weights sit transposed in shared memory so that the
 // four outputs computed together read 32 contiguous bytes per k (two LDS.128 warp broadcasts per 4 FMAs); input and
 // output tiles are staged through shared memory so that global accesses are coalesced.
-template <int HP>
+template <int HP, bool TANH>      // TANH: act may be B7_ACT_TANH (tanh kept out of the other instantiation, as in blr_dmma.cu)
 __global__ void __launch_bounds__(128)
 mlp_layer_kernel(const double* __restrict__ in, long long M, int h_in, int h_out, const double* __restrict__ W,
-                 const double* __restrict__ bias, int relu, double* __restrict__ out) {
+                 const double* __restrict__ bias, int act, double* __restrict__ out) {
   extern __shared__ __align__(16) double sh[];
   const int ho4 = (h_out + 3) & ~3;
   double* Wt = sh;                          // [HP][ho4]  (Wt[k][j] = W[j][k], zero padded)
@@ -442,7 +442,8 @@ mlp_layer_kernel(const double* __restrict__ in, long long M, int h_in, int h_out
       a2 = fma(w23.x, x[k], a2);
       a3 = fma(w23.y, x[k], a3);
     }
-    if (relu) { a0 = a0 > 0.0 ? a0 : 0.0; a1 = a1 > 0.0 ? a1 : 0.0; a2 = a2 > 0.0 ? a2 : 0.0; a3 = a3 > 0.0 ? a3 : 0.0; }
+    if (act == B7_ACT_RELU) { a0 = a0 > 0.0 ? a0 : 0.0; a1 = a1 > 0.0 ? a1 : 0.0; a2 = a2 > 0.0 ? a2 : 0.0; a3 = a3 > 0.0 ? a3 : 0.0; }
+    else if (TANH && act == B7_ACT_TANH) { a0 = tanh(a0); a1 = tanh(a1); a2 = tanh(a2); a3 = tanh(a3); }
     if (j < h_out) tile[tid * ldo + j] = a0;
     if (j + 1 < h_out) tile[tid * ldo + j + 1] = a1;
     if (j + 2 < h_out) tile[tid * ldo + j + 2] = a2;
@@ -453,16 +454,19 @@ mlp_layer_kernel(const double* __restrict__ in, long long M, int h_in, int h_out
 }
 
 template <int HP>
-int launch_mlp_layer(b7_ctx* ctx, const double* in, int64_t M, int h_in, int h_out, const double* W, const double* b, int relu,
+int launch_mlp_layer(b7_ctx* ctx, const double* in, int64_t M, int h_in, int h_out, const double* W, const double* b, int act,
                      double* out) {
   const int ho4 = (h_out + 3) & ~3, wmax = (h_in | 1) > (h_out | 1) ? (h_in | 1) : (h_out | 1);
   const size_t smem = ((size_t)HP * ho4 + ho4 + 128 * (size_t)wmax) * 8;
   static bool done[16] = {false};
   if (!done[ctx->device & 15]) {
-    B7_CUDA(cudaFuncSetAttribute(mlp_layer_kernel<HP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    B7_CUDA(cudaFuncSetAttribute(mlp_layer_kernel<HP, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    B7_CUDA(cudaFuncSetAttribute(mlp_layer_kernel<HP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     done[ctx->device & 15] = true;
   }
-  mlp_layer_kernel<HP><<<(unsigned)((M + 127) / 128), 128, smem, ctx->stream>>>(in, M, h_in, h_out, W, b, relu, out);
+  const unsigned blocks = (unsigned)((M + 127) / 128);
+  if (act == B7_ACT_TANH) mlp_layer_kernel<HP, true><<<blocks, 128, smem, ctx->stream>>>(in, M, h_in, h_out, W, b, act, out);
+  else mlp_layer_kernel<HP, false><<<blocks, 128, smem, ctx->stream>>>(in, M, h_in, h_out, W, b, act, out);
   b7_count(ctx);
   B7_CUDA(cudaGetLastError());
   return 0;
@@ -514,10 +518,25 @@ bool mlp_tiles_enabled() {
 
 }  // namespace
 
+int b7_check_act(const char* what, int n_layers, const int* act) {
+  if (!act) { b7_set_error("%s: null activation codes", what); return B7_ERR_ARG; }
+  for (int l = 0; l < n_layers; ++l)
+    if (act[l] != B7_ACT_NONE && act[l] != B7_ACT_RELU && act[l] != B7_ACT_TANH) {
+      b7_set_error("%s: unknown activation code %d after layer %d (B7_ACT_NONE, B7_ACT_RELU or B7_ACT_TANH)", what, act[l], l);
+      return B7_ERR_ARG;
+    }
+  return 0;
+}
+
 extern "C" {
 
 int b7_mlp_features(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, const double* const* W, const double* const* b,
                     int relu_last, b7_grid** out) {
+  return b7_mlp_features_act(ctx, in, n_layers, dims, W, b, b7_relu_codes(n_layers, relu_last).data(), out);
+}
+
+int b7_mlp_features_act(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, const double* const* W, const double* const* b,
+                        const int* act, b7_grid** out) {
   if (!ctx || !in || !out || n_layers < 1 || !dims || !W || !b || dims[0] != in->d) {
     b7_set_error("mlp_features: bad arguments (dims[0] must equal the grid's dims)");
     return B7_ERR_ARG;
@@ -526,6 +545,7 @@ int b7_mlp_features(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, con
   if (in->ctx != ctx) { b7_set_error("mlp_features: the grid lives on another context / device"); return B7_ERR_ARG; }
   for (int l = 0; l <= n_layers; ++l)
     if (dims[l] < 1 || dims[l] > 64) { b7_set_error("mlp_features: layer widths must be in [1, 64] (got %d)", dims[l]); return B7_ERR_ARG; }
+  B7_CHECK(b7_check_act("mlp_features", n_layers, act));
   B7_CUDA(cudaSetDevice(ctx->device));
   const int64_t M = in->rows;
   double* feat = nullptr;
@@ -535,7 +555,7 @@ int b7_mlp_features(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, con
     B7_CHECK(dw.upload(n_layers, dims, W, b));
     B7_CHECK(dalloc(ctx, &feat, (size_t)std::max<int64_t>(M, 1) * dims[n_layers]));
     StageTimer t(ctx, ST_BLR);
-    int rc_t = mlp_tiles_enabled() ? b7_launch_dngo_tiles(ctx, in->X, M, n_layers, dims, dw.W.data(), dw.b.data(), relu_last, nullptr, nullptr, nullptr,
+    int rc_t = mlp_tiles_enabled() ? b7_launch_dngo_tiles(ctx, in->X, M, n_layers, dims, dw.W.data(), dw.b.data(), act, nullptr, nullptr, nullptr,
                                                           0, 0, 0, nullptr, nullptr, feat)
                                    : 1;
     t.stop(1);
@@ -562,17 +582,16 @@ int b7_mlp_features(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, con
     if ((rc = dalloc(ctx, &dW, (size_t)hi * ho)) || (rc = dalloc(ctx, &db, (size_t)ho)) || (rc = dalloc(ctx, &dst, (size_t)std::max<int64_t>(M, 1) * ho))) break;
     cudaMemcpyAsync(dW, W[l], (size_t)hi * ho * 8, cudaMemcpyHostToDevice, ctx->stream);
     cudaMemcpyAsync(db, b[l], (size_t)ho * 8, cudaMemcpyHostToDevice, ctx->stream);
-    const int relu = (l < n_layers - 1) || relu_last;
     if (M > 0) {
       switch ((hi + 7) / 8) {
-        case 1: rc = launch_mlp_layer<8>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
-        case 2: rc = launch_mlp_layer<16>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
-        case 3: rc = launch_mlp_layer<24>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
-        case 4: rc = launch_mlp_layer<32>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
-        case 5: rc = launch_mlp_layer<40>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
-        case 6: rc = launch_mlp_layer<48>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
-        case 7: rc = launch_mlp_layer<56>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
-        default: rc = launch_mlp_layer<64>(ctx, cur, M, hi, ho, dW, db, relu, dst); break;
+        case 1: rc = launch_mlp_layer<8>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
+        case 2: rc = launch_mlp_layer<16>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
+        case 3: rc = launch_mlp_layer<24>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
+        case 4: rc = launch_mlp_layer<32>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
+        case 5: rc = launch_mlp_layer<40>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
+        case 6: rc = launch_mlp_layer<48>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
+        case 7: rc = launch_mlp_layer<56>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
+        default: rc = launch_mlp_layer<64>(ctx, cur, M, hi, ho, dW, db, act[l], dst); break;
       }
     }
     cudaStreamSynchronize(ctx->stream);
@@ -753,7 +772,7 @@ int b7_blr_predict(b7_blr* blr, int s, const double* Z1, int64_t M, double* mean
 // shared body of b7_blr_score (n_layers = 0: `features` already holds the basis) and b7_dngo_score (the basis is
 // evaluated tile by tile in front of the head and never stored)
 static int blr_score_impl(b7_blr* blr, b7_grid* features, int n_layers, const int* dims, const double* const* W, const double* const* b,
-                          int relu_last, int kind, double tradeoff, int bound, double sign, double fmin, double* score_host, int64_t* argmax,
+                          const int* act, int kind, double tradeoff, int bound, double sign, double fmin, double* score_host, int64_t* argmax,
                           int64_t* argmax_original, double* best, int64_t* nan_count) {
   if (!blr || !features || (kind != B7_SCORE_EI && kind != B7_SCORE_CB) || (n_layers == 0 && features->d != blr->D)) {
     b7_set_error("blr_score: bad arguments (feature dims %d vs D %d)", features ? features->d : -1, blr ? blr->D : -1);
@@ -794,7 +813,7 @@ static int blr_score_impl(b7_blr* blr, b7_grid* features, int n_layers, const in
       int chunk = 4;
       for (int c0 = 0; c0 < S && rc == 0;) {
         const int sc_ = std::min(chunk, S - c0);
-        rc = b7_launch_dngo_tiles(ctx, features->X, M, n_layers, dims, dw.W.data(), dw.b.data(), relu_last, blr->Linv + (size_t)c0 * D * D,
+        rc = b7_launch_dngo_tiles(ctx, features->X, M, n_layers, dims, dw.W.data(), dw.b.data(), act, blr->Linv + (size_t)c0 * D * D,
                                   blr->w + (size_t)c0 * D, blr->par + (size_t)c0 * 4, D, sc_, M, mom + (size_t)c0 * M,
                                   mom + (size_t)(S + c0) * M, nullptr);
         if (rc == 1 && chunk > 1 && c0 == 0) { chunk /= 2; rc = 0; continue; }
@@ -841,18 +860,26 @@ static int blr_score_impl(b7_blr* blr, b7_grid* features, int n_layers, const in
 
 int b7_blr_score(b7_blr* blr, b7_grid* features, int kind, double tradeoff, int bound, double sign, double fmin,
                  double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count) {
-  return blr_score_impl(blr, features, 0, nullptr, nullptr, nullptr, 0, kind, tradeoff, bound, sign, fmin, score_host, argmax, argmax_original,
+  return blr_score_impl(blr, features, 0, nullptr, nullptr, nullptr, nullptr, kind, tradeoff, bound, sign, fmin, score_host, argmax, argmax_original,
                         best, nan_count);
 }
 
 int b7_dngo_score(b7_blr* blr, b7_grid* grid, int n_layers, const int* dims, const double* const* W, const double* const* b, int relu_last,
                   int kind, double tradeoff, int bound, double sign, double fmin, double* score_host, int64_t* argmax,
                   int64_t* argmax_original, double* best, int64_t* nan_count) {
+  return b7_dngo_score_act(blr, grid, n_layers, dims, W, b, b7_relu_codes(n_layers, relu_last).data(), kind, tradeoff, bound, sign, fmin,
+                           score_host, argmax, argmax_original, best, nan_count);
+}
+
+int b7_dngo_score_act(b7_blr* blr, b7_grid* grid, int n_layers, const int* dims, const double* const* W, const double* const* b,
+                      const int* act, int kind, double tradeoff, int bound, double sign, double fmin, double* score_host, int64_t* argmax,
+                      int64_t* argmax_original, double* best, int64_t* nan_count) {
   if (!grid || n_layers < 1 || !dims || !W || !b || dims[0] != grid->d || !blr || dims[n_layers] != blr->D) {
     b7_set_error("dngo_score: bad arguments (dims[0] must equal the grid's dims, dims[n_layers] the head's D)");
     return B7_ERR_ARG;
   }
-  return blr_score_impl(blr, grid, n_layers, dims, W, b, relu_last, kind, tradeoff, bound, sign, fmin, score_host, argmax, argmax_original, best,
+  B7_CHECK(b7_check_act("dngo_score", n_layers, act));
+  return blr_score_impl(blr, grid, n_layers, dims, W, b, act, kind, tradeoff, bound, sign, fmin, score_host, argmax, argmax_original, best,
                         nan_count);
 }
 

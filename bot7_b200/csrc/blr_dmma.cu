@@ -1,10 +1,11 @@
-// DNGO candidate pass on the FP64 tensor pipe: (optional) ReLU MLP basis followed by the BLR head, tile by tile.
+// DNGO candidate pass on the FP64 tensor pipe: (optional) MLP basis (ReLU / tanh / no activation per layer) followed by the
+// BLR head, tile by tile.
 //
 // Replaces, for the candidate grid, what models/dngo.lua:155-174 does in 32-row Lua minibatches: Z1 = basis(X_hid)
 // (:165-171) and predictor:predict(Z0, Y0, Z1, ...) (:174).  One CTA works on tiles of 128 candidates that never
 // leave shared memory between the layers:
 //     act_0 = the tile's rows of the input grid (X, or precomputed features)
-//     act_l+1 = act(W_l act_l + b_l)                      l = 0 .. n_layers-1   (nn.Linear + ReLU)
+//     act_l+1 = act(W_l act_l + b_l)                      l = 0 .. n_layers-1   (nn.Linear + nn.ReLU / nn.Tanh / nothing)
 //     v = L_A^-1 phi,  var = |v|^2 + 1/beta,  mean = m + w^T phi                 per (alpha_p, beta) draw
 // Every product is a DMMA m8n8k4 fragment product: the weights (and, for the head, [L_A^-1 ; w^T] as one matrix whose
 // last row yields the mean) sit in shared memory for the whole launch with a leading dimension = 4 mod 16 doubles
@@ -40,7 +41,8 @@ __host__ __device__ inline int ld_of(int width) {
 struct Plan {
   int n_layers;                 // MLP layers before the head
   int width[MAXL + 1];          // width[0] = input width, width[l + 1] = output of layer l
-  int relu[MAXL];
+  int relu[MAXL];               // 1: ReLU after layer l
+  int tanh[MAXL];               // 1: tanh after layer l (dngo_tile_kernel<true> only)
   int w_off[MAXL];              // offsets (doubles) of the staged weights / biases in shared memory
   int b_off[MAXL];
   int head_off;                 // [S][rows_pad][ld(D)] head matrices
@@ -141,6 +143,9 @@ __device__ __forceinline__ void tile_mma(const double* __restrict__ A, int lda, 
   }
 }
 
+// TANH: some layer has B7_ACT_TANH.  The tanh pass is compiled only into that instantiation, so that a stack without Tanh runs
+// the instructions it ran before activation codes existed (the same SASS, register count and stack frame).
+template <bool TANH>
 __global__ void __launch_bounds__(THREADS, 2)
 dngo_tile_kernel(const double* __restrict__ in, long long M, Plan pl, Ptrs pt, const double* __restrict__ Linv, const double* __restrict__ wv,
                  const double* __restrict__ par, int D, long long ld_out, double* __restrict__ mean, double* __restrict__ var,
@@ -243,6 +248,18 @@ dngo_tile_kernel(const double* __restrict__ in, long long M, Plan pl, Ptrs pt, c
           }
       }
       __syncwarp();                                    // a warp only reads the 16 candidates it wrote
+      if (TANH && pl.tanh[l]) {
+        // a second pass over the warp's 16 x ho outputs in shared memory, one element per lane and step: tanh (libdevice,
+        // DESIGN.md section 4.5) inlined once rather than in each of the 32 unrolled slots of the loop above, and no lane
+        // idles while ho is not a multiple of 8
+        int cc = lane / ho, j = lane - cc * ho;
+        while (cc < 16) {
+          double* p = out + cc * lda + j;
+          *p = tanh(*p);
+          for (j += 32; j >= ho && cc < 16; j -= ho) ++cc;
+        }
+        __syncwarp();
+      }
       X = out;
       ldx = lda;
     }
@@ -307,7 +324,8 @@ dngo_tile_kernel(const double* __restrict__ in, long long M, Plan pl, Ptrs pt, c
 }
 
 // Plans the shared memory of one launch; returns 1 if the shapes do not fit the tile kernel.
-int plan_tiles(int n_layers, const int* dims, int relu_last, int D, int S, Plan* plan, size_t* smem_bytes) {
+// act: n_layers B7_ACT_* codes (checked by the caller); nullptr plans the shared memory only.
+int plan_tiles(int n_layers, const int* dims, const int* act, int D, int S, Plan* plan, size_t* smem_bytes) {
   if (n_layers > MAXL) return 1;
   Plan pl = {};
   pl.n_layers = n_layers;
@@ -321,7 +339,8 @@ int plan_tiles(int n_layers, const int* dims, int relu_last, int D, int S, Plan*
   if (S > 0 && (D != dims[n_layers] || D + 1 > 64)) return 1;
   for (int l = 0; l < n_layers; ++l) {
     const int rows = (dims[l + 1] + 7) / 8 * 8;
-    pl.relu[l] = (l < n_layers - 1 || relu_last) ? 1 : 0;
+    pl.relu[l] = act && act[l] == B7_ACT_RELU;
+    pl.tanh[l] = act && act[l] == B7_ACT_TANH;
     pl.w_off[l] = off; off += rows * ld_of(dims[l]);
     pl.b_off[l] = off; off += rows;
   }
@@ -347,18 +366,18 @@ int plan_tiles(int n_layers, const int* dims, int relu_last, int D, int S, Plan*
 bool b7_dngo_tiles_fit(int n_layers, const int* dims, int D) {
   Plan pl;
   size_t smem;
-  return n_layers >= 1 && plan_tiles(n_layers, dims, 0, D, 1, &pl, &smem) == 0;
+  return n_layers >= 1 && plan_tiles(n_layers, dims, nullptr, D, 1, &pl, &smem) == 0;
 }
 
 // Plans the shared memory, uploads nothing (all pointers are device pointers) and launches.  Returns 1 if the shapes
 // do not fit the tile kernel (the caller then uses the per-candidate kernels of blr.cu).
 int b7_launch_dngo_tiles(b7_ctx* ctx, const double* in, int64_t M, int n_layers, const int* dims, const double* const* W_dev,
-                         const double* const* b_dev, int relu_last, const double* Linv, const double* w, const double* par, int D, int S,
+                         const double* const* b_dev, const int* act, const double* Linv, const double* w, const double* par, int D, int S,
                          int64_t ld_out, double* mean, double* var, double* feat_out) {
   if (M <= 0) return 0;
   Plan pl;
   size_t smem;
-  if (plan_tiles(n_layers, dims, relu_last, D, S, &pl, &smem)) return 1;
+  if (plan_tiles(n_layers, dims, act, D, S, &pl, &smem)) return 1;
   Ptrs pt = {};
   for (int l = 0; l < n_layers; ++l) {
     pt.W[l] = W_dev[l];
@@ -366,13 +385,17 @@ int b7_launch_dngo_tiles(b7_ctx* ctx, const double* in, int64_t M, int n_layers,
   }
   static bool done[16] = {false};
   if (!done[ctx->device & 15]) {
-    B7_CUDA(cudaFuncSetAttribute(dngo_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    B7_CUDA(cudaFuncSetAttribute(dngo_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    B7_CUDA(cudaFuncSetAttribute(dngo_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
     done[ctx->device & 15] = true;
   }
+  bool tanh_any = false;
+  for (int l = 0; l < n_layers; ++l) tanh_any = tanh_any || pl.tanh[l];
   const int64_t n_tiles = (M + TC - 1) / TC;
   const int per_sm = smem <= 110 * 1024 ? 2 : 1;
   const int grid = (int)std::min<int64_t>(n_tiles, (int64_t)ctx->sm_count * per_sm);
-  dngo_tile_kernel<<<grid, THREADS, smem, ctx->stream>>>(in, M, pl, pt, Linv, w, par, D, ld_out, mean, var, feat_out);
+  if (tanh_any) dngo_tile_kernel<true><<<grid, THREADS, smem, ctx->stream>>>(in, M, pl, pt, Linv, w, par, D, ld_out, mean, var, feat_out);
+  else dngo_tile_kernel<false><<<grid, THREADS, smem, ctx->stream>>>(in, M, pl, pt, Linv, w, par, D, ld_out, mean, var, feat_out);
   b7_count(ctx);
   B7_CUDA(cudaGetLastError());
   return 0;

@@ -531,6 +531,13 @@ int b7_blr_fit_multi(b7_comm* c, const double* Z0, const double* y, int N, int D
 int b7_dngo_score_multi(b7_comm* c, b7_blr** blrs, b7_grid** grids, int n_layers, const int* dims, const double* const* W,
                         const double* const* b, int relu_last, int kind, double tradeoff, int bound, double sign, double fmin,
                         double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count) {
+  return b7_dngo_score_multi_act(c, blrs, grids, n_layers, dims, W, b, b7_relu_codes(n_layers, relu_last).data(), kind, tradeoff, bound,
+                                 sign, fmin, score_host, argmax, argmax_original, best, nan_count);
+}
+
+int b7_dngo_score_multi_act(b7_comm* c, b7_blr** blrs, b7_grid** grids, int n_layers, const int* dims, const double* const* W,
+                            const double* const* b, const int* act, int kind, double tradeoff, int bound, double sign, double fmin,
+                            double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count) {
   if (!c || !blrs || !grids || n_layers < 1 || !dims || !W || !b || (kind != B7_SCORE_EI && kind != B7_SCORE_CB)) {
     b7_set_error("dngo_score_multi: bad arguments");
     return B7_ERR_ARG;
@@ -551,20 +558,21 @@ int b7_dngo_score_multi(b7_comm* c, b7_blr** blrs, b7_grid** grids, int n_layers
       return B7_ERR_STATE;
     }
   }
-  // an empty shard launches nothing and would not notice: check the shapes here, for every rank alike
+  // an empty shard launches nothing and would not notice: check the shapes and the activation codes here, for every rank alike
   if (!b7_dngo_tiles_fit(n_layers, dims, dims[n_layers])) {
     b7_set_error("dngo_score: layer shapes do not fit the tile kernel (widths <= 63, at most 4 layers)");
     return B7_ERR_ARG;
   }
+  B7_CHECK(b7_check_act("dngo_score_multi", n_layers, act));
   if (c->world == 1)
-    return b7_dngo_score(blrs[0], grids[0], n_layers, dims, W, b, relu_last, kind, tradeoff, bound, sign, fmin, score_host, argmax,
+    return b7_dngo_score_act(blrs[0], grids[0], n_layers, dims, W, b, act, kind, tradeoff, bound, sign, fmin, score_host, argmax,
                          argmax_original, best, nan_count);
   std::vector<double> tb((size_t)n, NAN);
   std::vector<int64_t> ti((size_t)n, 0), tn((size_t)n, 0), off((size_t)n, 0);
   for (int i = 1; i < n; ++i) off[i] = off[i - 1] + grids[i - 1]->rows;
   int rc = for_each_local(c, [&](int i) {
     int64_t o = 0;
-    int rc_ = b7_dngo_score(blrs[i], grids[i], n_layers, dims, W, b, relu_last, kind, tradeoff, bound, sign, fmin,
+    int rc_ = b7_dngo_score_act(blrs[i], grids[i], n_layers, dims, W, b, act, kind, tradeoff, bound, sign, fmin,
                             score_host ? score_host + off[i] : nullptr, nullptr, &o, &tb[i], &tn[i]);
     ti[i] = o > 0 ? o + grids[i]->row_base : 0;      // local original row + the shard's first row: global, 1-based
     return rc_;

@@ -311,10 +311,19 @@ class BLRFactors:
             pass
 
 
-def mlp_features(grid, weights, biases, relu_last=True, ctx=None):
+def act_codes(act, n):
+    """n activation codes (L.ACT_NONE / ACT_RELU / ACT_TANH, one per layer) as a C int array; an unknown code is the library's
+    to refuse."""
+    if len(act) != n:
+        raise ValueError(f"act: {len(act)} codes for {n} layers")
+    return (C.c_int * n)(*[int(a) for a in act])
+
+
+def mlp_features(grid, weights, biases, relu_last=True, ctx=None, act=None):
     """DNGO basis on the device (models/dngo.lua:164-171 without the 32-row minibatch loop and without
-    the host round trip of Z1): ReLU MLP forward of a DeviceGrid, returns a DeviceGrid of features.
-    weights[l]: (h_out x h_in) like torch nn.Linear.weight; biases[l]: (h_out,)."""
+    the host round trip of Z1): MLP forward of a DeviceGrid, returns a DeviceGrid of features.
+    weights[l]: (h_out x h_in) like torch nn.Linear.weight; biases[l]: (h_out,).
+    act: one code per layer (b7_mlp_features_act); None is the relu_last form (b7_mlp_features)."""
     from .grids import DeviceGrid
     ctx = ctx or grid.ctx
     Ws = [L.as_f64(w) for w in weights]
@@ -324,14 +333,19 @@ def mlp_features(grid, weights, biases, relu_last=True, ctx=None):
     Wp = (C.POINTER(C.c_double) * n)(*[L.dptr(w) for w in Ws])
     bp = (C.POINTER(C.c_double) * n)(*[L.dptr(b) for b in bs])
     out = C.c_void_p()
-    L.check(L.lib().b7_mlp_features(ctx.handle, grid.handle, n, dims, Wp, bp, int(bool(relu_last)), C.byref(out)), "b7_mlp_features")
+    if act is None:
+        L.check(L.lib().b7_mlp_features(ctx.handle, grid.handle, n, dims, Wp, bp, int(bool(relu_last)), C.byref(out)), "b7_mlp_features")
+    else:
+        L.check(L.lib().b7_mlp_features_act(ctx.handle, grid.handle, n, dims, Wp, bp, act_codes(act, n), C.byref(out)),
+                "b7_mlp_features_act")
     return DeviceGrid(out, ctx)
 
 
 def dngo_score(blr, grid, weights, biases, relu_last=True, kind=L.SCORE_EI, tradeoff=0.0, bound=0, sign=-1.0, fmin=0.0,
-               want_scores=False):
+               want_scores=False, act=None):
     """dngo:predict + score + argmax over a device grid in one pass (b7_dngo_score; models/dngo.lua:155-174): the basis is
     evaluated in front of the BLR head tile by tile, the feature matrix Z1 is never stored.
+    act: one code per layer (b7_dngo_score_act); None is the relu_last form.
     Returns (scores or None, argmax (compacted), argmax_original, best, nan_count)."""
     Ws = [L.as_f64(w) for w in weights]
     bs = [L.as_f64(b).reshape(-1) for b in biases]
@@ -341,8 +355,12 @@ def dngo_score(blr, grid, weights, biases, relu_last=True, kind=L.SCORE_EI, trad
     bp = (C.POINTER(C.c_double) * n)(*[L.dptr(b) for b in bs])
     sc = np.empty(grid.rows()) if want_scores else None
     am, amo, best, nn = C.c_int64(), C.c_int64(), C.c_double(), C.c_int64()
-    L.check(L.lib().b7_dngo_score(blr.handle, grid.handle, n, dims, Wp, bp, int(bool(relu_last)), kind, tradeoff, bound, sign, fmin,
-                                  L.dptr(sc), C.byref(am), C.byref(amo), C.byref(best), C.byref(nn)), "b7_dngo_score")
+    if act is None:
+        L.check(L.lib().b7_dngo_score(blr.handle, grid.handle, n, dims, Wp, bp, int(bool(relu_last)), kind, tradeoff, bound, sign, fmin,
+                                      L.dptr(sc), C.byref(am), C.byref(amo), C.byref(best), C.byref(nn)), "b7_dngo_score")
+    else:
+        L.check(L.lib().b7_dngo_score_act(blr.handle, grid.handle, n, dims, Wp, bp, act_codes(act, n), kind, tradeoff, bound, sign, fmin,
+                                          L.dptr(sc), C.byref(am), C.byref(amo), C.byref(best), C.byref(nn)), "b7_dngo_score_act")
     return sc, am.value, amo.value, best.value, nn.value
 
 

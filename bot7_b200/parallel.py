@@ -217,9 +217,10 @@ class Comm:
             self._L.lib().b7_blr_free(h)
 
     def dngo_score(self, blrs, grids, weights, biases, relu_last=True, kind=0, tradeoff=0.0, bound=0, sign=-1.0, fmin=0.0,
-                   want_scores=False):
+                   want_scores=False, act=None):
         """b7_dngo_score_multi -> (best, argmax (global, compacted), argmax_original, nan_count, scores of the local shards or None).
-        weights[l]: (h_out x h_in) like torch nn.Linear.weight; biases[l]: (h_out,)."""
+        weights[l]: (h_out x h_in) like torch nn.Linear.weight; biases[l]: (h_out,).
+        act: one code per layer (b7_dngo_score_multi_act); None is the relu_last form."""
         L = self._L
         Ws = [L.as_f64(w) for w in weights]
         bs = [L.as_f64(b).reshape(-1) for b in biases]
@@ -230,9 +231,15 @@ class Comm:
         rows = sum(int(L.lib().b7_grid_rows(g.handle)) for g in grids)
         sc = np.empty(rows) if want_scores else None
         am, amo, best, nn = C.c_int64(), C.c_int64(), C.c_double(), C.c_int64()
-        L.check(L.lib().b7_dngo_score_multi(self.handle, (C.c_void_p * self.n_local)(*blrs), self._handles(grids), n, dims, Wp, bp,
-                                            int(bool(relu_last)), kind, tradeoff, bound, sign, fmin, L.dptr(sc), C.byref(am), C.byref(amo),
-                                            C.byref(best), C.byref(nn)), "b7_dngo_score_multi")
+        if act is None:
+            L.check(L.lib().b7_dngo_score_multi(self.handle, (C.c_void_p * self.n_local)(*blrs), self._handles(grids), n, dims, Wp, bp,
+                                                int(bool(relu_last)), kind, tradeoff, bound, sign, fmin, L.dptr(sc), C.byref(am),
+                                                C.byref(amo), C.byref(best), C.byref(nn)), "b7_dngo_score_multi")
+        else:
+            from .models import act_codes
+            L.check(L.lib().b7_dngo_score_multi_act(self.handle, (C.c_void_p * self.n_local)(*blrs), self._handles(grids), n, dims, Wp,
+                                                    bp, act_codes(act, n), kind, tradeoff, bound, sign, fmin, L.dptr(sc), C.byref(am),
+                                                    C.byref(amo), C.byref(best), C.byref(nn)), "b7_dngo_score_multi_act")
         return best.value, am.value, amo.value, nn.value, sc
 
     def close(self):

@@ -32,6 +32,7 @@ enum { B7_KERNEL_ARDSE = 0, B7_KERNEL_MATERN52 = 1 };           /* bots/bayesopt
 enum { B7_SCORE_EI = 0, B7_SCORE_CB = 1 };                       /* scores/init.lua */
 enum { B7_BOUND_LOWER = 0, B7_BOUND_UPPER = 1 };                 /* scores/confidence_bound.lua:32 */
 enum { B7_FIT_PREDICT = 0, B7_FIT_LOGML_ONLY = 1, B7_FIT_DEFER = 2 }; /* flags of b7_gp_fit */
+enum { B7_ACT_NONE = 0, B7_ACT_RELU = 1, B7_ACT_TANH = 2 };         /* activation after a Linear of the DNGO basis */
 enum { B7_ERR_ARG = -1, B7_ERR_CUDA = -2, B7_ERR_STATE = -3, B7_ERR_NOMEM = -4, B7_ERR_NCCL = -5 };
 
 int         b7_version(void);
@@ -146,12 +147,18 @@ int b7_score_moments(b7_ctx* ctx, int kind, const double* mean, const double* va
 /* ---- DNGO head: replaces bayes_linear:predict called from models/dngo.lua:174 -----------------
  * hyp: S x 3 rows [log alpha_p, log beta, m] (oracle/SPEC.md). */
 /* DNGO basis functions (models/dngo.lua:155-171: X -> output of the last hidden layer of the trained network):
- * ReLU MLP forward in fp64 on a device-resident grid.  dims[0..n_layers] are the widths (dims[0] = grid dims, each
+ * Linear/ReLU MLP forward in fp64 on a device-resident grid.  dims[0..n_layers] are the widths (dims[0] = grid dims, each
  * <= 64), W[l] is dims[l+1] x dims[l] row-major (torch nn.Linear.weight), b[l] has dims[l+1] entries; every layer is
  * followed by ReLU (the last one only if relu_last).  The result is a new device grid of features that inherits the
  * removed rows of the input grid and feeds b7_blr_score. */
 int b7_mlp_features(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, const double* const* W,
                     const double* const* b, int relu_last, b7_grid** out);
+/* Same, with one activation per layer instead of relu_last: act[l] (n_layers entries) follows layer l, B7_ACT_NONE (nothing,
+ * nn.Linear alone), B7_ACT_RELU (nn.ReLU, max(0, x)) or B7_ACT_TANH (nn.Tanh, fp64 tanh within 2 ulp).  An unknown code is
+ * B7_ERR_ARG before any device work.  b7_mlp_features is this call with B7_ACT_RELU for the inner layers and
+ * relu_last ? B7_ACT_RELU : B7_ACT_NONE for the last one. */
+int b7_mlp_features_act(b7_ctx* ctx, b7_grid* in, int n_layers, const int* dims, const double* const* W,
+                        const double* const* b, const int* act, b7_grid** out);
 int b7_blr_fit(b7_ctx* ctx, const double* Z0, const double* y, int N, int D, const double* hyp, int S,
                b7_blr** out, int* info);
 /* Same features and responses, new S x 3 rows [log alpha_p, log beta, m], every device buffer reused: the density the
@@ -174,6 +181,10 @@ int b7_blr_score(b7_blr* blr, b7_grid* features, int kind, double tradeoff, int 
 int b7_dngo_score(b7_blr* blr, b7_grid* grid, int n_layers, const int* dims, const double* const* W,
                   const double* const* b, int relu_last, int kind, double tradeoff, int bound, double sign, double fmin,
                   double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count);
+/* b7_dngo_score with one activation code per layer (act as in b7_mlp_features_act) */
+int b7_dngo_score_act(b7_blr* blr, b7_grid* grid, int n_layers, const int* dims, const double* const* W,
+                      const double* const* b, const int* act, int kind, double tradeoff, int bound, double sign, double fmin,
+                      double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count);
 void b7_blr_free(b7_blr* blr);
 
 /* ---- multi-GPU: candidate shards + draw-sharded fit (bots/bayesopt.lua:56-99 over config.bot.nGPU devices) ----
@@ -233,6 +244,11 @@ int  b7_blr_fit_multi(b7_comm* comm, const double* Z0, const double* y, int N, i
 int  b7_dngo_score_multi(b7_comm* comm, b7_blr** blrs, b7_grid** grids, int n_layers, const int* dims, const double* const* W,
                          const double* const* b, int relu_last, int kind, double tradeoff, int bound, double sign, double fmin,
                          double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count);
+/* b7_dngo_score_multi with one activation code per layer (act as in b7_mlp_features_act); an unknown code is B7_ERR_ARG on
+ * every rank, before any device work and without entering the all-gather, like the other argument checks. */
+int  b7_dngo_score_multi_act(b7_comm* comm, b7_blr** blrs, b7_grid** grids, int n_layers, const int* dims, const double* const* W,
+                             const double* const* b, const int* act, int kind, double tradeoff, int bound, double sign, double fmin,
+                             double* score_host, int64_t* argmax, int64_t* argmax_original, double* best, int64_t* nan_count);
 
 #ifdef __cplusplus
 }

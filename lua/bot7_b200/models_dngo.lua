@@ -1,8 +1,9 @@
 -- bot7.models.dngo with the hand-off of models/dngo.lua:155-174 routed to the GPU: the network update (trainer,
 -- :126-153) and every other method stay the parent's; what changes is how Z1 = basis(X_hid) and
 -- predictor:predict(Z0, Y0, Z1, nil, hyp, req) are evaluated for the candidate grid:
---   * the Linear / ReLU stack below the basis layer is read out of self.network and applied to the device grid by
---     b7_mlp_features (no 32-row minibatch loop, no host copy of Z1), the head is b7_blr_fit + b7_blr_predict;
+--   * the Linear / ReLU / Tanh stack below the basis layer is read out of self.network and applied to the device grid by
+--     b7_mlp_features (b7_mlp_features_act when it has Tanh or no-activation inner layers; no 32-row minibatch loop, no host
+--     copy of Z1), the head is b7_blr_fit + b7_blr_predict;
 --   * bots.bayesopt (bayesopt.lua) calls model:acquire(...), which fuses basis + head + score + argmax in one pass
 --     over the grid (b7_dngo_score) and never stores Z1; with config.bot.nGPU > 1 it calls model:acquire_multi(...), the
 --     same pass over the grid's shards (b7_blr_fit_multi + b7_dngo_score_multi).
@@ -21,29 +22,54 @@ end
 
 function dngo:class() return 'bot7.models.dngo' end
 
--- weights of the nn.Linear modules up to (and including) the basis layer: arrays for b7_mlp_features / b7_dngo_score
+-- weights of the nn.Linear modules up to (and including) the basis layer, with the activation that follows each one: arrays for
+-- b7_mlp_features(_act) / b7_dngo_score(_act).  Recognised: nn.Linear, nn.ReLU, nn.Tanh, and what is the identity in evaluation
+-- mode (nn.Identity; nn.Dropout in its v2 form, Torch7's default, or with p = 0).  Anything else -- another module, two
+-- activations after one Linear, an activation before the first Linear -- is an error naming the module and its position:
+-- the device would otherwise evaluate a different network than the host basis the head is fitted on.
+-- relu_last is set when the codes are the relu_last form (ReLU after every Linear but the last, ReLU or nothing after the
+-- last): such stacks keep calling the entries without _act.
+local ACT = {['nn.ReLU'] = 1, ['nn.Tanh'] = 2}                   -- B7_ACT_RELU, B7_ACT_TANH (B7_ACT_NONE = 0)
+
 function dngo:basis_stack()
-  local Ws, bs, dims, relu_last = {}, {}, {}, false
+  local Ws, bs, dims, codes = {}, {}, {}, {}
+  local acted = false                                            -- an activation already follows the last Linear
   for idx = 1, self.network:size() do
     local mod = self.network:get(idx)
-    if mod.weight then
-      assert(torch.type(mod) == 'nn.Linear', 'bot7_b200.models.dngo: the basis must be a Linear/ReLU stack (nnTools/builder.lua:133-159)')
+    local t   = torch.type(mod)
+    local where = string.format("module %d of the network (%s)", idx, t)
+    if t == 'nn.Linear' then
       Ws[#Ws + 1] = mod.weight:contiguous():double()         -- h_out x h_in, like torch nn.Linear.weight
       bs[#bs + 1] = mod.bias:contiguous():double()
       if #dims == 0 then dims[1] = mod.weight:size(2) end
       dims[#dims + 1] = mod.weight:size(1)
-      relu_last = false
-    elseif torch.type(mod) == 'nn.ReLU' then
-      relu_last = true
+      codes[#codes + 1] = 0
+      acted = false
+    elseif ACT[t] then
+      if #Ws == 0 then error('bot7_b200.models.dngo: ' .. where .. ' comes before the first nn.Linear of the basis', 2) end
+      if acted then error('bot7_b200.models.dngo: ' .. where .. ' is a second activation after one nn.Linear', 2) end
+      codes[#codes] = ACT[t]
+      acted = true
+    elseif t == 'nn.Identity' or (t == 'nn.Dropout' and (mod.v2 or (mod.p or 0) == 0)) then
+      -- the identity in evaluation mode (host_basis runs the network after :evaluate())
+    elseif t == 'nn.Dropout' then
+      error('bot7_b200.models.dngo: ' .. where .. ' is a v1 Dropout with p > 0, which scales by 1 - p in evaluation mode; ' ..
+            'the basis takes nn.Linear, nn.ReLU, nn.Tanh, nn.Identity and v2 nn.Dropout', 2)
+    else
+      error('bot7_b200.models.dngo: ' .. where .. ' is not supported in the basis; it takes nn.Linear, nn.ReLU, nn.Tanh, ' ..
+            'nn.Identity and v2 nn.Dropout', 2)
     end
     if mod == self.basis then break end
   end
   local n   = #Ws
+  local relu_form = n > 0 and codes[n] ~= 2
+  for l = 1, n - 1 do relu_form = relu_form and codes[l] == 1 end
   local cd  = ffi.new('int[?]', n + 1, dims)
   local cW  = ffi.new('const double*[?]', n)
   local cb  = ffi.new('const double*[?]', n)
   for l = 1, n do cW[l - 1] = Ws[l]:data(); cb[l - 1] = bs[l]:data() end
-  return {n = n, dims = cd, W = cW, b = cb, relu_last = relu_last and 1 or 0, keep = {Ws, bs}, zDim = dims[#dims]}
+  return {n = n, dims = cd, W = cW, b = cb, relu_last = (codes[n] == 1) and 1 or 0, act = ffi.new('int[?]', n, codes),
+          relu_form = relu_form, codes = codes, keep = {Ws, bs}, zDim = dims[#dims]}
 end
 
 -- Z = basis(X) on the host for the (few) observations, through the network itself (models/dngo.lua:155-162)
@@ -168,7 +194,11 @@ function dngo:predict(X0, Y0, X1, hyp, req, skip)
   local gbox, fbox = ffi.new('b7_grid*[1]'), ffi.new('b7_grid*[1]')
   B.check(B.C.b7_grid_from_host(B.context(), X1:data(), M, X1:size(2), gbox), 'b7_grid_from_host')
   local grid = ffi.gc(gbox[0], B.C.b7_grid_free)
-  B.check(B.C.b7_mlp_features(B.context(), grid, st.n, st.dims, st.W, st.b, st.relu_last, fbox), 'b7_mlp_features')
+  if st.relu_form then
+    B.check(B.C.b7_mlp_features(B.context(), grid, st.n, st.dims, st.W, st.b, st.relu_last, fbox), 'b7_mlp_features')
+  else
+    B.check(B.C.b7_mlp_features_act(B.context(), grid, st.n, st.dims, st.W, st.b, st.act, fbox), 'b7_mlp_features_act')
+  end
   local feats = ffi.gc(fbox[0], B.C.b7_grid_free)
   local Z1 = torch.DoubleTensor(M, st.zDim)
   B.check(B.C.b7_grid_read(feats, 0, M, Z1:data()), 'b7_grid_read')
@@ -189,8 +219,13 @@ function dngo:acquire(X0, Y0, grid_dev, kind, tradeoff, bound, sign, skip)
   local st  = self:basis_stack()
   local argmax, orig = ffi.new('int64_t[1]'), ffi.new('int64_t[1]')
   local best, nans   = ffi.new('double[1]'), ffi.new('int64_t[1]')
-  B.check(B.C.b7_dngo_score(blr, grid_dev, st.n, st.dims, st.W, st.b, st.relu_last, kind, tradeoff, bound, sign, Y0:min(),
-                            nil, argmax, orig, best, nans), 'b7_dngo_score')
+  if st.relu_form then
+    B.check(B.C.b7_dngo_score(blr, grid_dev, st.n, st.dims, st.W, st.b, st.relu_last, kind, tradeoff, bound, sign, Y0:min(),
+                              nil, argmax, orig, best, nans), 'b7_dngo_score')
+  else
+    B.check(B.C.b7_dngo_score_act(blr, grid_dev, st.n, st.dims, st.W, st.b, st.act, kind, tradeoff, bound, sign, Y0:min(),
+                                  nil, argmax, orig, best, nans), 'b7_dngo_score_act')
+  end
   return tonumber(argmax[0]), best[0], tonumber(nans[0])
 end
 
@@ -208,10 +243,16 @@ function dngo:acquire_multi(X0, Y0, comm, grids, nGPU, kind, tradeoff, bound, si
   local st = self:basis_stack()
   local argmax, orig = ffi.new('int64_t[1]'), ffi.new('int64_t[1]')
   local best, nans   = ffi.new('double[1]'), ffi.new('int64_t[1]')
-  local rc = B.C.b7_dngo_score_multi(comm, blrs, grids, st.n, st.dims, st.W, st.b, st.relu_last, kind, tradeoff, bound, sign, Y0:min(),
-                                     nil, argmax, orig, best, nans)
+  local rc, what
+  if st.relu_form then
+    rc, what = B.C.b7_dngo_score_multi(comm, blrs, grids, st.n, st.dims, st.W, st.b, st.relu_last, kind, tradeoff, bound, sign,
+                                       Y0:min(), nil, argmax, orig, best, nans), 'b7_dngo_score_multi'
+  else
+    rc, what = B.C.b7_dngo_score_multi_act(comm, blrs, grids, st.n, st.dims, st.W, st.b, st.act, kind, tradeoff, bound, sign,
+                                           Y0:min(), nil, argmax, orig, best, nans), 'b7_dngo_score_multi_act'
+  end
   for g = 0, nGPU - 1 do B.C.b7_blr_free(blrs[g]) end
-  B.check(rc, 'b7_dngo_score_multi')
+  B.check(rc, what)
   return tonumber(argmax[0]), best[0], tonumber(nans[0])
 end
 
