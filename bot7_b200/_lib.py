@@ -20,6 +20,7 @@ BOUND_LOWER, BOUND_UPPER = 0, 1
 FIT_PREDICT, FIT_LOGML_ONLY, FIT_DEFER = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_TANH = 0, 1, 2
 PATH_FP64_DMMA, PATH_INT8_OZAKI = 0, 1
+ERR_ARG, ERR_CUDA, ERR_STATE = -1, -2, -3
 STAGES = ("sobol", "kbuild", "potrf", "trtri", "kstar", "posterior", "score", "blr")
 
 _p = C.c_void_p
@@ -56,6 +57,7 @@ SIGNATURES = {
     "b7_grid_free": (None, [_p]),
     "b7_gp_fit": (_i, [_p, _i, _dp, _dp, _i, _i, _dp, _i, _i, _i, _i, C.POINTER(_p), _ip, _dp, _dp]),
     "b7_gp_refit": (_i, [_p, _dp, _i, _ip, _dp, _dp]),
+    "b7_gp_slice_step": (_i, [_p, _dp, _dp, _d, _dp, _dp, _i, _d, _d, _d, _i, _dp, _ip, _ip, _dp]),
     "b7_gp_num_draws": (_i, [_p]),
     "b7_gp_num_obs": (_i, [_p]),
     "b7_gp_predict": (_i, [_p, _i, _dp, _l, _dp, _dp]),

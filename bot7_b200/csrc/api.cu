@@ -451,7 +451,7 @@ void b7_gp_free(b7_gp* gp) {
   if (!gp) return;
   cudaSetDevice(gp->ctx->device);
   cudaStreamSynchronize(gp->ctx->stream);
-  void* ptrs[] = {gp->X, gp->Xt, gp->y, gp->par, gp->fac, gp->facS, gp->sigma, gp->dinv, gp->dinvT, gp->beta, gp->alpha, gp->tt, gp->logdet, gp->info, gp->meta_dev};
+  void* ptrs[] = {gp->X, gp->Xt, gp->y, gp->par, gp->fac, gp->facS, gp->sigma, gp->dinv, gp->dinvT, gp->beta, gp->alpha, gp->tt, gp->logdet, gp->info, gp->meta_dev, gp->step_io};
   for (void* p : ptrs) dev_free(gp->ctx, p);
   if (gp->potrf_graph) cudaGraphExecDestroy(gp->potrf_graph);
   delete gp;
@@ -738,6 +738,46 @@ int b7_gp_refit(b7_gp* gp, const double* hyp, int flags, int* info, double* logm
   }
   B7_CUDA(cudaStreamSynchronize(ctx->stream));
   gp->ready = true;
+  return 0;
+}
+
+// One directed slice step in one launch (slice_step.cu): the random numbers go in, the new point comes out.
+int b7_gp_slice_step(b7_gp* gp, const double* x0, const double* dir, double log_u_level, const double* u_right,
+                     const double* u_shrink, int K, double width, double max_step, double prior_std, int prior_order,
+                     double* x1, int* n_shrink_used, int* n_evals, double* logp_x1) {
+  if (!gp || !x0 || !dir || !u_right || K < 0 || (K > 0 && !u_shrink) || !x1 || (prior_order != 0 && prior_order != 1)) {
+    b7_set_error("gp_slice_step: bad arguments");
+    return B7_ERR_ARG;
+  }
+  if (gp->N > B7_NB) {
+    b7_set_error("gp_slice_step: %d observations; the one-launch step takes at most %d", gp->N, B7_NB);
+    return B7_ERR_ARG;
+  }
+  if (!(width > 0.0) || !std::isfinite(width)) {
+    b7_set_error("gp_slice_step: width %g is not a finite positive number", width);
+    return B7_ERR_ARG;
+  }
+  b7_ctx* ctx = gp->ctx;
+  B7_CUDA(cudaSetDevice(ctx->device));
+  const int H = gp->d + 3;
+  std::vector<double> in((size_t)3 * H + K), out((size_t)H + 4);
+  std::copy(x0, x0 + H, in.begin());
+  std::copy(dir, dir + H, in.begin() + H);
+  std::copy(u_right, u_right + H, in.begin() + 2 * H);
+  if (K > 0) std::copy(u_shrink, u_shrink + K, in.begin() + 3 * H);
+  B7_CHECK(grow(ctx, &gp->step_io, &gp->step_io_bytes, (in.size() + out.size()) * sizeof(double)));
+  B7_CUDA(cudaMemcpyAsync(gp->step_io, in.data(), in.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  B7_CHECK(b7_launch_slice_step(gp, gp->step_io, K, log_u_level, width, max_step, prior_std, prior_order));
+  B7_CUDA(cudaMemcpyAsync(out.data(), gp->step_io + in.size(), out.size() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  B7_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (out[H + 3] != 0.0) {
+    b7_set_error("gp_slice_step: the %d shrink uniforms ran out; call again with more", K);
+    return B7_ERR_STATE;
+  }
+  std::copy(out.begin(), out.begin() + H, x1);
+  if (logp_x1) *logp_x1 = out[H];
+  if (n_shrink_used) *n_shrink_used = (int)out[H + 1];
+  if (n_evals) *n_evals = (int)out[H + 2];
   return 0;
 }
 

@@ -104,6 +104,8 @@ struct b7_gp {
   double* logdet = nullptr; // device S : sum log L_ii
   int* info = nullptr;      // device S
   double* meta_dev = nullptr;   // device S x 3 : (info, log ml, jitter) per draw, exchanged by the sharded fit
+  double* step_io = nullptr;    // device in / out of b7_gp_slice_step (grown on demand)
+  size_t step_io_bytes = 0;
   // single-factor Cholesky replayed as a CUDA graph from the second call with the same (first draw, count) on
   // (the slice sampler's density evaluations: same handle, new hyper-parameters in device memory)
   cudaGraphExec_t potrf_graph = nullptr;
@@ -186,6 +188,10 @@ int b7_launch_cov_batched(b7_ctx* ctx, int kernel, const double* A /* rows x d *
 int b7_launch_potrf(b7_gp* gp, int s0, int count);      // K -> L, beta, logdet, info for draws [s0,s0+count)
 int b7_launch_trtri(b7_gp* gp, int s0, int count);      // L -> L^-1 in place
 int b7_launch_alpha(b7_gp* gp, int s0, int count, bool from_inverse);   // alpha = L^-T beta (from L, or from L^-1)
+// slice_step.cu: one directed slice step of a fit with Np == 128; io = [x0 | dir | u_right] (H each), u_shrink (K), then
+// the outputs x1 (H), log p(x1), shrink uniforms used, evaluations, status (1: the K uniforms ran out)
+int b7_launch_slice_step(b7_gp* gp, double* io, int K, double log_u, double width, double max_step, double prior_std,
+                         int prior_order);
 // posterior.cu
 int b7_launch_untile(b7_ctx* ctx, const double* facT, double* out /* N x N row-major */, int Np, int N);
 int b7_launch_posterior(b7_ctx* ctx, const double* LinvT /* tiled */, const double* beta, int Np, const double* ksT /* tiled */,

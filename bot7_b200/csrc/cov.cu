@@ -13,7 +13,7 @@
 // (candidates) whose coordinates sit in shared memory and are read as warp broadcasts; every
 // store instruction writes 32 consecutive doubles.
 #include "b7_internal.h"
-#include "exp_neg.cuh"
+#include "cov_entry.cuh"
 
 namespace {
 
@@ -59,12 +59,7 @@ cov_kernel(const double* __restrict__ A, long long rows, long long rows_pad, int
         double t = (s_a[r][i] - b[i]) * s_w[i];
         r2 = fma(t, t, r2);
       }
-      if (KERNEL == B7_KERNEL_ARDSE) {
-        val = sf2 * exp_neg(-0.5 * r2, s_tab);
-      } else {
-        double rr = sqrt(r2), s5r = 2.23606797749978969641 * rr;
-        val = sf2 * ((1.0 + s5r + (5.0 / 3.0) * r2) * exp_neg(-s5r, s_tab));
-      }
+      val = cov_value<KERNEL>(r2, sf2, s_tab);
       if (is_kxx && row == k) val += diag_add;
     }
     if (tiled) {

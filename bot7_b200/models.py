@@ -16,8 +16,9 @@ import numpy as np
 
 from . import _lib as L
 from .samplers import slice as slice_sampler
-from .samplers import slice_speculative
+from .samplers import slice_device, slice_speculative
 
+DEVICE_STEP_MAX_N = 128    # b7_gp_slice_step: one 128 x 128 block
 KERNELS = {"ardse": L.KERNEL_ARDSE, "matern52": L.KERNEL_MATERN52, "matern_52": L.KERNEL_MATERN52}
 
 
@@ -63,6 +64,23 @@ class GPFactors:
         self.hyp = hyp
         self.info = np.array(list(info), dtype=np.int32)
         return self
+
+    def slice_step(self, x0, d_vec, log_u, u_right, u_shrink, width, max_step, prior_std, prior_order):
+        """One directed slice step on this handle's observations in one device call (b7_gp_slice_step, N <= 128) ->
+        (x1 (1 x H), shrink uniforms used, density evaluations, log p(x1)), or None when `u_shrink` ran out."""
+        H = self.d + 3
+        x0, d_vec, u_right = (L.as_f64(v).reshape(-1) for v in (x0, d_vec, u_right))
+        u_shrink = L.as_f64(u_shrink).reshape(-1)
+        if x0.size != H or d_vec.size != H or u_right.size != H:
+            raise ValueError(f"slice_step: the handle's hyper-parameter rows have H = {H} entries")
+        x1, used, evals, logp = np.empty((1, H)), C.c_int(), C.c_int(), C.c_double()
+        rc = L.lib().b7_gp_slice_step(self.handle, L.dptr(x0), L.dptr(d_vec), float(log_u), L.dptr(u_right), L.dptr(u_shrink),
+                                      u_shrink.size, float(width), float(max_step), float(prior_std), int(prior_order),
+                                      L.dptr(x1), C.byref(used), C.byref(evals), C.byref(logp))
+        if rc == L.ERR_STATE:
+            return None
+        L.check(rc, "b7_gp_slice_step")
+        return x1, used.value, evals.value, logp.value
 
     def predict(self, s, Xs):
         Xs = L.as_f64(Xs)
@@ -136,6 +154,9 @@ class gp_regressor:
         c.setdefault("init_noise", None)   # sigma_n^2; None: 1e-2, or 1e-6 with `noiseless`
         c.setdefault("speculative", True)  # batched density evaluations; the chain is identical either way
         c.setdefault("spec_width", 8)     # profiles/refit_vs_width_r01.json: 8 evaluations cost 1.0-2.1x one
+        # one device call per slice step (b7_gp_slice_step) for fits of up to 128 observations; the chain is identical, larger
+        # fits keep the route above
+        c.setdefault("device_step", False)
         self.config = c
         self.ctx = ctx
         self.rng = rng or np.random.default_rng(0)
@@ -212,6 +233,14 @@ class gp_regressor:
                 out.append(lp - 0.5 * float(np.sum((chunk[i] / sd) ** 2)))
         return out
 
+    def device_step(self, X, Y, x0, d_vec, log_u, u_right, u_shrink, width, max_step):
+        """One slice step in one device call on the single-slot handle of log_density (X, y resident); numpy's pairwise
+        order for the prior's sum, as log_density's np.sum."""
+        key = (np.asarray(X).tobytes(), np.asarray(Y).tobytes(), 1)
+        if self._density_key != key:
+            self.log_density(x0, X, Y)
+        return self._density.slice_step(x0, d_vec, log_u, u_right, u_shrink, width, max_step, self.config["prior_std"], 1)
+
     def sample_hypers(self, X, Y, _a=None, _b=None, single=False):
         """bots/bayesopt.lua:68,74: slice-sample the hyper-parameter posterior, keep the chain state."""
         if self.hyp is None:
@@ -219,8 +248,11 @@ class gp_regressor:
         n = 1 if single else int(self.config["nSamples"])
         out = np.empty((n, self.hyp.size))
         x = self.hyp.reshape(1, -1).copy()
+        device = self.config["device_step"] and np.atleast_2d(X).shape[0] <= DEVICE_STEP_MAX_N
         for i in range(n):
-            if self.config["speculative"]:
+            if device:
+                x = slice_device()(lambda *a: self.device_step(X, Y, *a), x, {"nSamples": 1}, None, rng=self.rng)
+            elif self.config["speculative"]:
                 x = slice_speculative()(lambda V, a: self.log_density_batch(V, X, Y), x, {"nSamples": 1}, None,
                                         rng=self.rng, width=int(self.config["spec_width"]))
             else:

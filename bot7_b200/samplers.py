@@ -6,6 +6,8 @@ here) and is not reproduced; the control flow is.
 """
 from __future__ import annotations
 
+import copy
+
 import numpy as np
 
 
@@ -225,3 +227,53 @@ class slice_speculative(slice):
             if done:
                 break
         return x0 + d_vec * dx
+
+
+class slice_device(slice):
+    """Same chain as `slice`, one device call per step: `step` runs the whole directed slice step (b7_gp_slice_step).
+
+    The generator stays on the host.  Each step pre-draws, from a copy of it, what the sequential sampler would consume in its
+    order -- H normals for the direction, one uniform for the level, H for the bracket, then `k` shrink uniforms -- and passes
+    the normalised direction, log U and the uniforms to `step(x0, d_vec, log_u, u_right, u_shrink, width, max_step)`, which
+    returns (x1, shrink uniforms used, density evaluations, log p(x1)), or None when the `k` shrink uniforms ran out (the step
+    is then made again from the same draws with twice as many).  The real generator then advances by exactly what the
+    sequential sampler would have drawn, so for a given generator the samples are bit-identical to `slice`.  The NaN exit
+    prints the reference's message; the shrink-to-zero exit ends the step the same way but is not reported.  Gibbs sweeps and
+    per-dimension `widths` stay on the other samplers.
+    """
+
+    def __call__(self, step, X0, opt=None, f_args=None, rng=None, k=16):
+        opt = self.configure(opt)
+        rng = rng or np.random.default_rng()
+        if opt.get("gibbs") or opt.get("widths") is not None or not opt["logspace"] or not opt["step_out"]:
+            raise NotImplementedError("the device step runs the log-space directed step with step-out and a scalar width")
+        X0 = np.atleast_2d(np.asarray(X0, dtype=np.float64))
+        X0 = np.tile(X0.copy(), (int(opt["nSamples"]), 1))
+        N, xDim = X0.shape
+        samples = np.empty((N, xDim))
+        self.calls = 0          # device calls (one per step, more when the shrink uniforms ran out)
+        self.evals = 0          # density evaluations
+        width = float(opt.get("width") or 1.0)
+        for n in range(N):
+            x0 = X0[n:n + 1]
+            while True:
+                r = copy.deepcopy(rng)
+                d_vec = r.standard_normal((1, xDim))
+                d_vec = d_vec / np.linalg.norm(d_vec)
+                log_u = float(np.log(r.random()))
+                u_right = r.random((1, xDim))
+                res = step(x0, d_vec, log_u, u_right, r.random(int(k)), width, float(opt["max_step"]))
+                self.calls += 1
+                if res is not None:
+                    break
+                k = 2 * int(k)
+            x1, used, evals, logp = res
+            self.evals += evals
+            if logp != logp:
+                print("Error: samplers.slice encountered a NaN")
+            rng.standard_normal((1, xDim))
+            rng.random()
+            rng.random((1, xDim))
+            rng.random(used)
+            samples[n] = x1
+        return samples

@@ -103,6 +103,19 @@ int b7_gp_fit(b7_ctx* ctx, int kernel, const double* X, const double* y, int N, 
  * evaluation of the slice sampler (samplers/slice.lua:100-103) with X and y resident.
  * flags: B7_FIT_PREDICT or B7_FIT_LOGML_ONLY. */
 int b7_gp_refit(b7_gp* gp, const double* hyp, int flags, int* info, double* logml, double* jitter);
+/* One directed slice step (samplers/slice.lua:92-168) on the density log p(y | h) + log p(h) of this handle's
+ * observations, in one launch, for N <= 128: every density is the value b7_gp_refit(B7_FIT_LOGML_ONLY) gives for that
+ * row at this N (-inf unless info == 0 and finite) minus 1/2 sum (h_i / prior_std)^2, summed in prior_order (0 sequential
+ * as Torch7, 1 numpy's pairwise sum).  The handle is only read (typically the one of B7_FIT_LOGML_ONLY); H = d + 3.
+ * The caller draws the step's random numbers in the reference's order and passes them in: the direction (normalised:
+ * dir), log U of the slice level, H uniforms of the bracket, then K shrink uniforms.  width: the scalar bracket width
+ * (opt.width), max_step: the step-out limit per side.  Out: x1 = x0 + dir * dx (H), the shrink uniforms consumed, the
+ * density evaluations made, log p(x1).  B7_ERR_ARG for N > 128 or a width that is not finite and positive;
+ * B7_ERR_STATE when the K shrink uniforms ran out (call again with the same numbers and a larger K). */
+int b7_gp_slice_step(b7_gp* gp, const double* x0 /* H */, const double* dir /* H, unit */, double log_u_level,
+                     const double* u_right /* H */, const double* u_shrink /* K */, int K, double width,
+                     double max_step, double prior_std, int prior_order, double* x1 /* H */, int* n_shrink_used,
+                     int* n_evals, double* logp_x1);
 int b7_gp_num_draws(b7_gp* gp);
 int b7_gp_num_obs(b7_gp* gp);
 /* model:predict(X_obs,Y_obs,X_hid,hyp,{mean,var}) for draw s (0-based): M x d host points ->

@@ -27,6 +27,9 @@ function model:__init(config)
   -- batched density evaluations through sampler_spec.lua: the chain of bot7.samplers.slice from the same generator state,
   -- in fewer device calls (false: the reference sampler, one evaluation per call)
   if config.speculative == nil then config['speculative'] = true end
+  -- one device call per slice step through sampler_device.lua (b7_gp_slice_step) for fits of up to 128 observations; the
+  -- same chain, larger fits keep the route above
+  if config.device_step == nil then config['device_step'] = false end
   -- declared initial state of the chain (model:init); gpTorch7's own values are unknown
   config['init_lengthscale'] = config.init_lengthscale or 0.5
   config['init_sigma_f']     = config.init_sigma_f or 1.0
@@ -131,14 +134,37 @@ function model:log_density(h, X, Y)
   return self:log_density_batch(self:parse_hypers(h), X, Y, 1)[1]
 end
 
+-- one slice step in one device call on the single-slot handle of log_density (X, y resident); Torch7's sequential order for
+-- the prior's sum.  Returns {x1, used, evals, logp}, or nil when the shrink uniforms ran out.
+function model:device_step(X, Y, x0, dir, log_u, u_right, u_shrink, width, max_step)
+  local slot = self._density and self._density[1]
+  if slot == nil or slot.X ~= X or slot.Y ~= Y then
+    self:log_density(x0, X, Y)
+    slot = self._density[1]
+  end
+  local H = x0:nElement()
+  local x1 = torch.DoubleTensor(1, H)
+  local used, evals, logp = ffi.new('int[1]'), ffi.new('int[1]'), ffi.new('double[1]')
+  local x0c, dirc, urc, usc = x0:contiguous():double(), dir:contiguous():double(), u_right:contiguous():double(), u_shrink:contiguous():double()
+  local rc = B.C.b7_gp_slice_step(slot.gp, x0c:data(), dirc:data(), log_u, urc:data(), usc:data(), usc:nElement(), width, max_step,
+                                  self.config.prior_std, 0, x1:data(), used, evals, logp)
+  if rc == B.C.B7_ERR_STATE then return nil end
+  B.check(rc, 'b7_gp_slice_step')
+  return {x1 = x1, used = used[0], evals = evals[0], logp = logp[0]}
+end
+
 ---------------- bots/bayesopt.lua:68,74: slice-sample the hyper-parameter posterior, keep the chain state.
 -- bot7.samplers.slice (samplers/slice.lua, unchanged) drives the chain; each f(x) is one density evaluation on the GPU.
 function model:sample_hypers(X, Y, _, _, single)
   if self.hyp == nil then self:init(X, Y) end
   local n    = single and 1 or self.config.nSamples
-  local spec = self.config.speculative and self.config.sampler == 'slice'
+  local dev  = self.config.device_step and self.config.sampler == 'slice' and X:size(1) <= 128
+  local spec = not dev and self.config.speculative and self.config.sampler == 'slice'
   local sampler, f
-  if spec then
+  if dev then
+    sampler = require('bot7_b200.sampler_device')()
+    f       = function(...) return self:device_step(X, Y, ...) end
+  elseif spec then
     sampler = require('bot7_b200.sampler_spec')()
     f       = function(V, args) return self:log_density_batch(V, X, Y) end
   else
@@ -148,7 +174,9 @@ function model:sample_hypers(X, Y, _, _, single)
   local out = torch.DoubleTensor(n, self.hyp:nElement())
   local x   = self.hyp:view(1, -1):clone()
   for i = 1, n do
-    if spec then
+    if dev then
+      x = sampler(f, x, {nSamples = 1}, nil)
+    elseif spec then
       x = sampler(f, x, {nSamples = 1}, nil, self.config.spec_width)
     else
       x = sampler(f, x, {nSamples = 1}, nil)
